@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host cores
+    python bench.py --gpus N --steps K --dump-outputs DIR    # + the outputs of the last timed step as DIR/*.npy
+
+The library is loaded as `python __graft_entry__.py build` left it (a missing or stale one is refused); the benchmark compiles nothing
+and writes nothing into the tree.
 
 Workload (BASELINE.json configs[4], SURVEY.md 8d "config 5"): 2^20 environments in total, split
 evenly over the N ranks (one process per GPU, no data-path collective -- environments are
@@ -31,6 +35,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the tree may be read-only where the benchmark runs: no __pycache__ next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -42,6 +47,8 @@ SOLVER = "motor rows eliminated (motor_solver=auto -> exact), PGS <= 50 sweeps o
 BYTES_PER_ENV_STEP = 621
 # fp32 instructions per lane-cycle the CUDA cores can retire: 128 lanes x 2 (FMA) per SM and clock
 FP32_FLOP_PER_SM_CLK = 256.0
+# environments whose outputs --dump-outputs writes: 2^17 x (56 + 3) float32 = 31 MB
+DUMP_ENVS = 1 << 17
 
 
 def workload_config(total, world):
@@ -215,6 +222,24 @@ def time_cuda(fn, iters, torch, dist, world, dev):
     return float(t.item())
 
 
+def dump_outputs(path, total, lo, hi, outs, rank, world, dist):
+    """--dump-outputs: obs / reward / done / ticks of the last timed step for a fixed sample of DUMP_ENVS global environment ids
+    (seed 0, ascending), as float32 `path`/<name>.npy written by rank 0 -- the whole batch would be 2^20 x 59 floats = 247 MB."""
+    import numpy as np
+    import torch
+    ids = np.sort(np.random.default_rng(0).choice(total, min(total, DUMP_ENVS), replace=False))
+    rows = torch.as_tensor(ids[(ids >= lo) & (ids < hi)] - lo, device=outs[0].device)
+    part = [t[rows].float().cpu().numpy() for t in outs]
+    parts = [part]
+    if world > 1:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(part, parts, dst=0)  # shards are contiguous and in rank order: the rows stay ascending
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        for i, name in enumerate(("obs", "reward", "done", "ticks")):
+            np.save(os.path.join(path, name + ".npy"), np.concatenate([p[i] for p in parts]))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -234,12 +259,11 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
 
     import __graft_entry__ as ge
-    if rank == 0:
-        ge.build()
-    if world > 1:
-        dist.barrier()
     from bullet_envs_b200 import SnakeVecEnv, _abi, default_params
     from bullet_envs_b200 import dist as sd
+    if _abi.LIB_PATH == ge.LIB and ge._stale(ge.LIB, ge.DEPS):
+        raise RuntimeError("%s is missing or older than its sources: run `python __graft_entry__.py build` first "
+                           "(the benchmark compiles nothing)" % ge.LIB)
 
     total = args.envs
     lo, hi = sd.shard_range(total, rank, world)
@@ -274,6 +298,8 @@ def run_ours(args):
     barrier()
     ms = e0.elapsed_time(e1)
     gpu_launches = env.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, total, lo, hi, (obs, rew, done, env.last_ticks), rank, world, dist)
     # per-launch kernel time on the launching stream (second pass, one event pair per launch) + tick statistics
     kt = []
     sweeps = 0.0
@@ -531,7 +557,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config4", action="store_true")
     ap.add_argument("--no-bullet-order", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write obs / reward / done / ticks of the last timed step (a fixed sample of "
+                                                          "%d environments) as DIR/<name>.npy, float32" % DUMP_ENVS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to this repo's arm (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     return run_reference(args) if args.impl == "reference" else run_ours(args)

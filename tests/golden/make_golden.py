@@ -154,6 +154,19 @@ def scenario_actions():
     return sc
 
 
+# merged-body tables of a URDF that tests/test_model_tables.py compares between the reference's snake/snake.urdf and snake_chain.urdf
+URDF_TABLES = ("joint_R0", "joint_t", "joint_axis", "joint_damping", "body_mass", "body_com", "body_inertia", "cyl_center", "cyl_axis",
+               "cyl_fric_R", "cyl_radius", "cyl_halflen", "cyl_end", "cyl_break", "height_pt", "fz_axis", "cyl_body", "height_body")
+
+
+def urdf_tables(path):
+    m = build_model(path)
+    out = {name: getattr(m, name) for name in URDF_TABLES}
+    out["motor_joint_indices"] = np.asarray(m.motor_joint_indices)
+    out["num_urdf_links"] = np.asarray(m.num_urdf_links)
+    return out
+
+
 # state edits applied to the (fake) simulator before a step: step -> (delta z of the base, delta vz of the base)
 INJECT = {"lifted": {0: (0.2, 0.0), 3: (0.0, 3.0), 5: (0.2, 0.0)}}
 
@@ -254,6 +267,11 @@ def main():
         print("raw single-env %-12s steps %d dones %d return %.4f" % (name, len(actions), int(np.sum(dn)), float(np.sum(rw))))
     path = os.path.join(ROOT, "tests", "golden", "reference_python_raw_single_env.npz")
     np.savez_compressed(path, **raw)
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+    # the model tables PyBullet's importer would build from the reference's own URDF (snake.py:93)
+    path = os.path.join(ROOT, "tests", "golden", "reference_urdf_model_tables.npz")
+    np.savez_compressed(path, **urdf_tables(os.path.join(REF, "snake", "snake.urdf")))
     print("wrote", path, os.path.getsize(path), "bytes")
 
 

@@ -6,7 +6,7 @@ import pytest
 
 from bullet_envs_b200.urdf_model import DEFAULT_URDF, ImportRules, build_model, dfs_order, parse_urdf
 
-REF_URDF = "/root/reference/snake/snake.urdf"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_urdf_model_tables.npz")
 
 
 def test_link_and_joint_counts_and_motor_indices(model):
@@ -71,14 +71,17 @@ def test_height_points_and_fz_axis(model):
     assert np.allclose(model.fz_axis, [-1, 0, 0], atol=1e-9) and model.root_mass == 1.0
 
 
-@pytest.mark.skipif(not os.path.exists(REF_URDF), reason="reference tree not mounted (GPU box)")
 def test_generated_urdf_equals_reference_urdf(model):
-    ref = build_model(REF_URDF)
-    for name in ("joint_R0", "joint_t", "joint_axis", "joint_damping", "body_mass", "body_com", "body_inertia", "cyl_center",
-                 "cyl_axis", "cyl_fric_R", "cyl_radius", "cyl_halflen", "cyl_end", "cyl_break", "height_pt", "fz_axis", "cyl_body",
-                 "height_body"):
-        assert np.array_equal(getattr(ref, name), getattr(model, name)), name
-    assert ref.motor_joint_indices == model.motor_joint_indices and ref.num_urdf_links == 50
+    """the tables of the physics-only snake_chain.urdf against those of the reference's snake/snake.urdf, stored by
+    tests/golden/make_golden.py (urdf_tables)"""
+    ref = np.load(GOLDEN)
+    names = ("joint_R0", "joint_t", "joint_axis", "joint_damping", "body_mass", "body_com", "body_inertia", "cyl_center",
+             "cyl_axis", "cyl_fric_R", "cyl_radius", "cyl_halflen", "cyl_end", "cyl_break", "height_pt", "fz_axis", "cyl_body",
+             "height_body")
+    assert sorted(ref.files) == sorted(names + ("motor_joint_indices", "num_urdf_links"))
+    for name in names:
+        assert np.array_equal(ref[name], getattr(model, name)), name
+    assert list(ref["motor_joint_indices"]) == model.motor_joint_indices and int(ref["num_urdf_links"]) == 50
 
 
 def test_ctypes_round_trip(model):
