@@ -1083,4 +1083,18 @@ cudaError_t snk_exact_launch_tick(const KParams& P, float* state, const float* t
     else snk_exact_tick_kernel<false><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, targets, counters, n, n_ticks);
     return cudaGetLastError();
 }
+
+#ifdef SNK_PHASE_CLOCKS
+// phase clocks of the current device (see ExPhaseClock): copies the [SNK_CLK_WARPS][SNK_CLK_PHASES] cycle sums to `out` (may be null), then
+// zeroes them when `reset` is set.  Synchronises the device.
+extern "C" int snk_phase_clocks(unsigned long long* out, int reset) {
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e == cudaSuccess && out) e = cudaMemcpyFromSymbol(out, snk_phase_clk, sizeof(snk_phase_clk));
+    if (e == cudaSuccess && reset) {
+        static unsigned long long zero[SNK_CLK_WARPS][SNK_CLK_PHASES];
+        e = cudaMemcpyToSymbol(snk_phase_clk, zero, sizeof(zero));
+    }
+    return (int)e;
+}
+#endif
 #endif // SNK_SCREEN

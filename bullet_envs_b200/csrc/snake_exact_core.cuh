@@ -458,6 +458,31 @@ struct ExCursor {
 
 struct ExTickOut { int iterations; int contacts; float height; float err2_next; };
 
+// Phase clocks (build variant -DSNK_PHASE_CLOCKS; tools/bench_phases.py reads them through snk_phase_clocks): lane 0 of every warp
+// adds the clock64() cycles the warp spends in each phase of ex_tick -- 0 pass 1, 1 rows + solver prologue, 2 solver, 3 pass 2 +
+// finish -- to row (global warp % SNK_CLK_WARPS) of snk_phase_clk.  The default build contains none of this.
+#if defined(SNK_PHASE_CLOCKS) && defined(__CUDACC__)
+#define SNK_CLK_WARPS 4096
+#define SNK_CLK_PHASES 4
+__device__ unsigned long long snk_phase_clk[SNK_CLK_WARPS][SNK_CLK_PHASES];
+#endif
+#if defined(SNK_PHASE_CLOCKS) && defined(__CUDA_ARCH__)
+struct ExPhaseClock {
+    long long t = clock64();
+    __device__ __forceinline__ void mark(int phase) {
+        const long long now = clock64();
+        if ((threadIdx.x & 31) == 0)
+            atomicAdd(&snk_phase_clk[((blockIdx.x * blockDim.x + threadIdx.x) >> 5) % SNK_CLK_WARPS][phase], (unsigned long long)(now - t));
+        t = now;
+    }
+};
+#define SNK_PHASE_START ExPhaseClock phase_clock;
+#define SNK_PHASE_MARK(k) phase_clock.mark(k);
+#else
+#define SNK_PHASE_START
+#define SNK_PHASE_MARK(k)
+#endif
+
 // -----------------------------------------------------------------------------------------------
 // One physics tick.  Returns the mean checkSnakeHeight z of the state at the START of the tick in
 // out->height; when that height already exceeds the threshold and `abort_on_height` is set, nothing is
@@ -469,6 +494,7 @@ template <bool CONE, class Rows>
 SNK_HD void ex_tick(const ExTables& T, const KParams& P, const Rows& R, ExEnv& e, bool active, bool abort_on_height, bool* aborted, ExTickOut* out) {
     const float dt = P.dt, inv_dt = P.inv_dt;
     const float p0z = e.pos[2];
+    SNK_PHASE_START
     // ------------------------------------------------------------------ pass 1: tip-ward
     ExCursor c;
     c.R = quat_to_m3(e.quat);
@@ -480,6 +506,10 @@ SNK_HD void ex_tick(const ExTables& T, const KParams& P, const Rows& R, ExEnv& e
     S3 J; J.xx = J.xy = J.xz = J.yy = J.yz = J.zz = 0.f;
     float hsum = 0.f, err2n = 0.f;
     unsigned act = 0u;
+    // what pass 2 needs of body i >= 1, kept by pass 1 in six float4 (local memory): (Iw.xx xy xz yy | Iw.yz zz, a.x a.y | a.z, p |
+    // cc, F.x | F.y F.z, N.x N.y | N.z) with a the world axis of joint i-1, p the frame origin and F, N the reference wrench of body i
+    float4 keep[NJ][6];
+    V3 ja = mk(0.f, 0.f, 0.f);
     float qn = slot(e, SNK_S_Q), qdn = slot(e, SNK_S_QD); // prefetched joint 0
 #pragma unroll 1
     for (int i = 0; i < NB; i++) {
@@ -499,11 +529,12 @@ SNK_HD void ex_tick(const ExTables& T, const KParams& P, const Rows& R, ExEnv& e
             vJ = vJ + cross(wJ, d);
             c.p = c.p + d;
             c.R = mul(c.R, joint_rot(T, j, q));
-            V3 a = mul(c.R, ld3(T.jax[j]));
+            const V3 a = mul(c.R, ld3(T.jax[j]));
             V3 wq = a * qd;
             c.al = c.al + a * qdd + cross(c.w, wq);
             c.w = c.w + wq;
             wJ = wJ + a * qds;
+            ja = a;
         }
         // ---- body i
         {
@@ -523,6 +554,12 @@ SNK_HD void ex_tick(const ExTables& T, const KParams& P, const Rows& R, ExEnv& e
             J.xx += Iw.xx + m * (c2 - cc.x * cc.x); J.yy += Iw.yy + m * (c2 - cc.y * cc.y); J.zz += Iw.zz + m * (c2 - cc.z * cc.z);
             J.xy += Iw.xy - m * cc.x * cc.y; J.xz += Iw.xz - m * cc.x * cc.z; J.yz += Iw.yz - m * cc.y * cc.z;
             hsum += p0z + c.p.z + c.R.m[6] * T.hpt[i][0] + c.R.m[7] * T.hpt[i][1] + c.R.m[8] * T.hpt[i][2];
+            if (i > 0) {
+                float4* k = keep[i - 1];
+                k[0] = make_float4(Iw.xx, Iw.xy, Iw.xz, Iw.yy); k[1] = make_float4(Iw.yz, Iw.zz, ja.x, ja.y);
+                k[2] = make_float4(ja.z, c.p.x, c.p.y, c.p.z); k[3] = make_float4(cc.x, cc.y, cc.z, F.x);
+                k[4] = make_float4(F.y, F.z, N.x, N.y);       k[5] = make_float4(N.z, 0.f, 0.f, 0.f);
+            }
         }
         // ---- contacts of body i (A.5 with deviation D1: lowest point of the extreme rim)
 #pragma unroll 1
@@ -553,6 +590,7 @@ SNK_HD void ex_tick(const ExTables& T, const KParams& P, const Rows& R, ExEnv& e
     out->err2_next = err2n;
     *aborted = abort_on_height && out->height > P.hthr;
     const bool commit = active && !*aborted;
+    SNK_PHASE_MARK(0)
 
     // ------------------------------------------------------------------ free rigid motion about C
     const float invM = T.inv_mtot, M = T.mtot;
@@ -625,6 +663,7 @@ SNK_HD void ex_tick(const ExTables& T, const KParams& P, const Rows& R, ExEnv& e
         for (int k = 0; k < NC; k++) R.clr_lf(k);
         R.fence_st();
     }
+    SNK_PHASE_MARK(1)
 
     // ------------------------------------------------------------------ projected Gauss-Seidel
     // The only serial dependence is the 6-vector (dw, dV); everything else of a row (loads, impulse
@@ -761,6 +800,7 @@ SNK_UNROLL(SNK_UNROLL_F)
     }
     out->iterations = sweeps;
     out->contacts = ex_popc(act);
+    SNK_PHASE_MARK(2)
 
     // ------------------------------------------------------------------ new base velocity
     // rigid field after the solve: angular wf + dw, velocity VC + dV at C; base origin = field at -hc
@@ -777,6 +817,13 @@ SNK_UNROLL(SNK_UNROLL_F)
     const V3 wN = mul(R0, wb), vN = mul(R0, vb);
 
     // ------------------------------------------------------------------ pass 2: base-ward, torques
+    // Newton-Euler is linear in the accelerations, and the true ones differ from the reference ones of pass 1 by the base's
+    // (a0, al0): the wrench of body i is the reference wrench plus  m (a0 + al0 x cc)  and  Iw al0.  Pass 2 therefore walks no
+    // kinematics: it reads back what pass 1 kept of every body.  Only the torques (and, through them, the energy term of the
+    // reward) depend on pass 2; they differ from a recomputed wrench at round-off.
+#ifdef SNK_PASS2_RECOMPUTE
+    // (build variant: the earlier pass 2, which walks the chain back and recomputes every wrench; the reference of
+    // tests/test_gpu_setup_passes.py)
     {
         V3 SF = mk(0.f, 0.f, 0.f), SN = SF; // suffix wrench about the base origin
 #pragma unroll 1
@@ -828,6 +875,44 @@ SNK_UNROLL(SNK_UNROLL_F)
             c.acc = c.acc - cross(c.al, d) - cross(c.w, wxd);
         }
     }
+#else
+    {
+        V3 SF = mk(0.f, 0.f, 0.f), SN = SF; // suffix wrench about the base origin
+#pragma unroll 1
+        for (int j = NJ - 1; j >= 0; j--) {
+            const int i = j + 1;
+            const float4 k0 = keep[j][0], k1 = keep[j][1], k2 = keep[j][2], k3 = keep[j][3], k4 = keep[j][4], k5 = keep[j][5];
+            const float q = slot(e, SNK_S_Q + j), qd = slot(e, SNK_S_QD + j), tg = R.tgt(j);
+            float qds = P.kp * (tg - q) * inv_dt;
+            qds = ex_clamp(qds, P.maxvel);
+            // wrench of body i with the true accelerations
+            S3 Iw; Iw.xx = k0.x; Iw.xy = k0.y; Iw.xz = k0.z; Iw.yy = k0.w; Iw.yz = k1.x; Iw.zz = k1.y;
+            const V3 a = mk(k1.z, k1.w, k2.x), p = mk(k2.y, k2.z, k2.w), cc = mk(k3.x, k3.y, k3.z);
+            const V3 F = mk(k3.w, k4.x, k4.y) + (a0 + cross(al0, cc)) * T.mass[i];
+            const V3 N = mk(k4.z, k4.w, k5.x) + mul(Iw, al0);
+            SF = SF + F;
+            SN = SN + cross(cc, F) + N;
+#pragma unroll 1
+            for (int k = T.cstart[i]; k < T.cstart[i + 1]; k++) { // a separated contact has a zero record: zero force
+                float4 x0, x1, x2, x3;
+                R.ld16(k, x0, x1, x2, x3);
+                R.fence16(x0, x1, x2, x3);
+                // contact force n ln + d1 la + d2 lb with d2 = (x2.x, -x1.y, x2.y); explicit fma so that every row-storage
+                // instantiation rounds alike
+                V3 f = mk(fmaf(x2.x, x3.y, x1.y * x3.x), fmaf(-x1.y, x3.y, x1.z * x3.x), fmaf(x2.y, x3.y, fmaf(x1.w, x3.x, x0.x))) * inv_dt;
+                V3 r = mk(x0.y + hc.x, x0.z + hc.y, x1.x + hc.z); // back to the base origin
+                SF = SF - f;
+                SN = SN - cross(r, f);
+            }
+            const float tau = dot(a, SN - cross(p, SF)) + T.jdamp[j] * qd;
+            if (commit) {
+                slot(e, SNK_S_TAU + j) = tau;
+                slot(e, SNK_S_QD + j) = qds;
+                slot(e, SNK_S_Q + j) = q + qds * dt;
+            }
+        }
+    }
+#endif
 
     // ------------------------------------------------------------------ finish: Fz, base integration
     {   // reaction force of joint 0 (kdl_dummy_root -> base), z of link `base` (snake.py:202-206)
@@ -857,6 +942,7 @@ SNK_UNROLL(SNK_UNROLL_F)
         e.quat[0] = x * in; e.quat[1] = y * in; e.quat[2] = z * in; e.quat[3] = w * in;
     }
     }
+    SNK_PHASE_MARK(3)
 }
 
 // mean z of the checkSnakeHeight points (snake.py:237-245) of the current state: a z-only walk
