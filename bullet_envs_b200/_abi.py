@@ -111,6 +111,9 @@ def load_library():
     lib.snk_rollout_linear.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp, vp]
     lib.snk_set_manifold.argtypes = [vp, ctypes.c_int, ctypes.c_double]
     lib.snk_manifold_stats.argtypes = [vp, P(i64)]
+    lib.snk_get_manifold_cache.argtypes = [vp, vp, vp]
+    lib.snk_set_manifold_cache.argtypes = [vp, vp, vp]
+    lib.snk_clear_manifold.argtypes = [vp, vp, vp]
     lib.snk_gae.argtypes = [ctypes.c_int, vp, vp, vp, vp, ctypes.c_double, ctypes.c_double, vp, vp, i32, i64, vp]
     lib.snk_observe.argtypes = [vp, vp, vp]
     lib.snk_self_clearance.argtypes = [vp, vp, vp]

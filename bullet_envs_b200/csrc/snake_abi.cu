@@ -46,6 +46,14 @@ size_t snk_man_scratch_bytes();
 size_t snk_man_cache_floats();
 cudaError_t snk_man_launch_step(const KParams& P, float* state, float* tgt_scratch, float* cache, void* scratch, float warm, const float* actions, float* obs,
                                 float* rew, uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st);
+cudaError_t snk_man_launch_step_trace(const KParams& P, float* state, float* tgt_scratch, float* cache, void* scratch, float warm, const float* actions,
+                                      float* obs, float* rew, uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, float* tick_obs,
+                                      float* tick_links, cudaStream_t st);
+cudaError_t snk_man_launch_rollout(const KParams& P, float* state, float* tgt_scratch, float* cache, void* scratch, float warm, const float* weights,
+                                   const float* mean, const float* inv_std, const float* noise, int n_steps, float* returns, float* trace,
+                                   unsigned long long* counters, int64_t n, cudaStream_t st);
+cudaError_t snk_man_launch_clear(float* cache, const uint8_t* mask, int64_t n, cudaStream_t st);
+cudaError_t snk_man_launch_check(const float* cache, int64_t n, unsigned long long* bad, cudaStream_t st);
 // generalised advantage estimation (snake_gae.cu)
 cudaError_t snk_launch_gae(const float* rewards, const uint8_t* dones, const float* values, const float* next_value, float gamma, float tau,
                            float* returns, float* advantages, int T, int64_t n, cudaStream_t st);
@@ -87,6 +95,7 @@ struct snk_handle {
     bool manifold;
     float* man_cache;             // device [n][MAN_STRIDE]
     void* man_scratch;            // device, snk_man_scratch_bytes()
+    unsigned long long* man_bad;  // device, 1 word: result of the count-word check of snk_set_manifold_cache
     float man_warm;
     // staging for the *_host entry points (allocated on first use)
     cudaEvent_t ev_dev;           // recorded after every state-touching launch on a caller stream; the *_host entry points
@@ -233,7 +242,7 @@ int snk_create(const snk_model* model, const snk_params* params, int64_t n_envs,
     if (err == cudaSuccess) err = cudaDeviceSynchronize();
     if (err != cudaSuccess) {
         if (h->exact) snk_exact_release();
-        cudaFree(h->man_cache); cudaFree(h->man_scratch);
+        cudaFree(h->man_cache); cudaFree(h->man_scratch); cudaFree(h->man_bad);
     cudaFree(h->T); cudaFree(h->state); cudaFree(h->counters); cudaFree(h->bucket); cudaFree(h->order); cudaFree(h->split_buf); cudaFree(h->tgt);
         delete h;
         return fail(SNK_E_CUDA, "snk_create: %s", cudaGetErrorString(err));
@@ -258,6 +267,7 @@ int snk_destroy(snk_handle* h) {
     for (int c = 0; c < h->n_ev_chunk; c++) cudaEventDestroy(h->ev_chunk[c]);
     if (h->exact) snk_exact_release();
     cudaFree(h->T); cudaFree(h->state); cudaFree(h->counters); cudaFree(h->bucket); cudaFree(h->order); cudaFree(h->split_buf); cudaFree(h->roll_queue); cudaFree(h->tgt);
+    cudaFree(h->man_cache); cudaFree(h->man_scratch); cudaFree(h->man_bad);
     delete h;
     return 0;
 }
@@ -302,11 +312,12 @@ int snk_step_trace(snk_handle* h, const float* actions_dev, float* obs_dev, floa
     if (!h || !actions_dev || !obs_dev || !rew_dev || !done_dev || !ticks_dev)
         return fail(SNK_E_ARG, "snk_step_trace: null pointer (ticks_dev is required: it says how many trace rows are valid)%s");
     if (!aligned16(actions_dev) || !aligned16(obs_dev)) return fail(SNK_E_ARG, "snk_step_trace: actions and obs must be 16-byte aligned%s");
-    if (h->manifold) return fail(SNK_E_ARG, "snk_step_trace: not available with persistent manifolds (snk_set_manifold); use snk_step%s");
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaMemsetAsync(h->counters, 0, NCOUNTERS * sizeof(unsigned long long), st));
-    if (h->exact) CU(snk_exact_launch_step_trace(h->P, h->state, h->tgt, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters, h->n, tick_obs_dev,
+    if (h->manifold) CU(snk_man_launch_step_trace(h->P, h->state, h->tgt, h->man_cache, h->man_scratch, h->man_warm, actions_dev, obs_dev, rew_dev, done_dev,
+                                                  ticks_dev, h->counters, h->n, tick_obs_dev, tick_links_dev, st));
+    else if (h->exact) CU(snk_exact_launch_step_trace(h->P, h->state, h->tgt, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters, h->n, tick_obs_dev,
                                                  tick_links_dev, st));
     else CU(snk_pgs_launch_step(h->T, h->P, h->state, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters, h->n, st, tick_obs_dev,
                                 tick_links_dev));
@@ -320,9 +331,16 @@ int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mea
     if (!h || !weights_dev || !returns_dev || n_steps < 1) return fail(SNK_E_ARG, "snk_rollout_linear: bad argument%s");
     if (!h->exact) return fail(SNK_E_ARG, "snk_rollout_linear: only with the exact motor solver (motor force = inf, kd = 1)%s");
     if (!aligned16(weights_dev)) return fail(SNK_E_ARG, "snk_rollout_linear: weights must be 16-byte aligned%s");
-    if (h->manifold) return fail(SNK_E_ARG, "snk_rollout_linear: not available with persistent manifolds (snk_set_manifold); use snk_step%s");
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
+    if (h->manifold) { // one environment per thread for the whole rollout: no ready queue, no hand-out order
+        CU(cudaMemsetAsync(h->counters, 0, NCOUNTERS * sizeof(unsigned long long), st));
+        CU(snk_man_launch_rollout(h->P, h->state, h->tgt, h->man_cache, h->man_scratch, h->man_warm, weights_dev, mean_dev, inv_std_dev, noise_dev, n_steps,
+                                  returns_dev, obs_trace_dev, h->counters, h->n, st));
+        h->launches++;
+        mark_device_work(h, st);
+        return 0;
+    }
     const size_t qlen = (size_t)h->n * (size_t)(n_steps > 1 ? n_steps - 1 : 1);
     if (qlen > h->roll_queue_len) { // grow the ready queue (first call, or a longer rollout than before)
         CU(cudaStreamSynchronize(st));
@@ -347,22 +365,63 @@ int snk_set_manifold(snk_handle* h, int on, double warm_start) {
     CU(cudaSetDevice(h->device));
     CU(cudaDeviceSynchronize()); // the caches of a step in flight are about to be cleared or freed
     if (!on) {
-        cudaFree(h->man_cache); cudaFree(h->man_scratch);
-        h->man_cache = nullptr; h->man_scratch = nullptr; h->manifold = false;
+        cudaFree(h->man_cache); cudaFree(h->man_scratch); cudaFree(h->man_bad);
+        h->man_cache = nullptr; h->man_scratch = nullptr; h->man_bad = nullptr; h->manifold = false;
         return 0;
     }
     const size_t cache_bytes = (size_t)h->n * snk_man_cache_floats() * sizeof(float);
     if (!h->man_cache) {
-        if (cudaMalloc(&h->man_cache, cache_bytes) != cudaSuccess || cudaMalloc(&h->man_scratch, snk_man_scratch_bytes()) != cudaSuccess) {
+        if (cudaMalloc(&h->man_cache, cache_bytes) != cudaSuccess || cudaMalloc(&h->man_scratch, snk_man_scratch_bytes()) != cudaSuccess ||
+            cudaMalloc(&h->man_bad, sizeof(unsigned long long)) != cudaSuccess) {
             cudaGetLastError();
-            cudaFree(h->man_cache); cudaFree(h->man_scratch);
-            h->man_cache = nullptr; h->man_scratch = nullptr; h->manifold = false;
+            cudaFree(h->man_cache); cudaFree(h->man_scratch); cudaFree(h->man_bad);
+            h->man_cache = nullptr; h->man_scratch = nullptr; h->man_bad = nullptr; h->manifold = false;
             return fail(SNK_E_NOMEM, "snk_set_manifold: out of device memory (4 224 B per environment + 388 MB of row tables)%s");
         }
     }
     CU(cudaMemset(h->man_cache, 0, cache_bytes)); // empty caches, like a freshly loaded world
     h->man_warm = (float)warm_start;
     h->manifold = true;
+    return 0;
+}
+
+int snk_get_manifold_cache(snk_handle* h, float* cache_dev, void* stream) {
+    if (!h || !cache_dev) return fail(SNK_E_ARG, "snk_get_manifold_cache: null pointer%s");
+    if (!h->manifold) return fail(SNK_E_ARG, "snk_get_manifold_cache: persistent manifolds are off (snk_set_manifold)%s");
+    CU(cudaSetDevice(h->device));
+    CU(cudaMemcpyAsync(cache_dev, h->man_cache, (size_t)h->n * SNK_MAN_STRIDE * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    mark_device_work(h, (cudaStream_t)stream);
+    return 0;
+}
+
+int snk_set_manifold_cache(snk_handle* h, const float* cache_dev, void* stream) {
+    if (!h || !cache_dev) return fail(SNK_E_ARG, "snk_set_manifold_cache: null pointer%s");
+    if (!h->manifold) return fail(SNK_E_ARG, "snk_set_manifold_cache: persistent manifolds are off (snk_set_manifold)%s");
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned long long bad = 0;
+    CU(cudaMemsetAsync(h->man_bad, 0, sizeof bad, st));
+    CU(snk_man_launch_check(cache_dev, h->n, h->man_bad, st));
+    h->launches++;
+    CU(cudaMemcpyAsync(&bad, h->man_bad, sizeof bad, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (bad) {
+        static thread_local char msg[128];
+        snprintf(msg, sizeof msg, "%llu environment(s) with a point count that is not an integer in 0..4", bad);
+        return fail(SNK_E_ARG, "snk_set_manifold_cache: %s; the caches are unchanged", msg);
+    }
+    CU(cudaMemcpyAsync(h->man_cache, cache_dev, (size_t)h->n * SNK_MAN_STRIDE * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    mark_device_work(h, st);
+    return 0;
+}
+
+int snk_clear_manifold(snk_handle* h, const uint8_t* mask_dev, void* stream) {
+    if (!h) return fail(SNK_E_ARG, "snk_clear_manifold: null handle%s");
+    if (!h->manifold) return fail(SNK_E_ARG, "snk_clear_manifold: persistent manifolds are off (snk_set_manifold)%s");
+    CU(cudaSetDevice(h->device));
+    CU(snk_man_launch_clear(h->man_cache, mask_dev, h->n, (cudaStream_t)stream));
+    h->launches++;
+    mark_device_work(h, (cudaStream_t)stream);
     return 0;
 }
 

@@ -906,6 +906,10 @@ cudaError_t snk_exact_configure(const ExTables* host_tables) {
     if (e == cudaSuccess) e = set_smem(snk_hyb_rollout_kernel<false>, sizeof(StepSmemH));
     if (e == cudaSuccess) e = set_smem(snk_man_step_kernel<true>, MAN_RING_BYTES);
     if (e == cudaSuccess) e = set_smem(snk_man_step_kernel<false>, MAN_RING_BYTES);
+    if (e == cudaSuccess) e = set_smem(snk_man_step_trace_kernel<true>, MAN_RING_BYTES);
+    if (e == cudaSuccess) e = set_smem(snk_man_step_trace_kernel<false>, MAN_RING_BYTES);
+    if (e == cudaSuccess) e = set_smem(snk_man_rollout_kernel<true>, MAN_RING_BYTES);
+    if (e == cudaSuccess) e = set_smem(snk_man_rollout_kernel<false>, MAN_RING_BYTES);
     // MAN_MINB CTAs x MAN_RING_BYTES of ring per SM and the rest of the 256 KB as L1 (state records, contact caches, local arrays): the
     // carveout is requested explicitly, otherwise it depends on which kernel ran before (a larger one costs L1: 3 CTAs x 60 KB ran 277 ms
     // against 228 ms for 2 x 60 KB at 262 144 environments)
@@ -913,8 +917,10 @@ cudaError_t snk_exact_configure(const ExTables* host_tables) {
         int pct = (int)((MAN_MINB * (MAN_RING_BYTES + 1024) * 100 + 233471) / 233472);
         if (getenv("SNK_MAN_CARVEOUT")) pct = atoi(getenv("SNK_MAN_CARVEOUT"));
         if (pct > 100) pct = 100;
-        if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)snk_man_step_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)snk_man_step_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+        const void* man_kernels[] = {(const void*)snk_man_step_kernel<true>, (const void*)snk_man_step_kernel<false>, (const void*)snk_man_step_trace_kernel<true>,
+                                     (const void*)snk_man_step_trace_kernel<false>, (const void*)snk_man_rollout_kernel<true>, (const void*)snk_man_rollout_kernel<false>};
+        for (const void* k : man_kernels)
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     }
     if (e != cudaSuccess) return e;
     int per_sm = 0;
@@ -1018,6 +1024,44 @@ cudaError_t snk_man_launch_step(const KParams& P, float* state, float* tgt_scrat
     dim3 grid((unsigned)(want < full ? want : full)), block(MAN_THREADS);
     if (P.cone) snk_man_step_kernel<true><<<grid, block, MAN_RING_BYTES, st>>>(P, state, tgt_scratch, cache, (float4*)scratch, warm, actions, obs, rew, done, ticks, counters, n);
     else snk_man_step_kernel<false><<<grid, block, MAN_RING_BYTES, st>>>(P, state, tgt_scratch, cache, (float4*)scratch, warm, actions, obs, rew, done, ticks, counters, n);
+    return cudaGetLastError();
+}
+
+cudaError_t snk_man_launch_step_trace(const KParams& P, float* state, float* tgt_scratch, float* cache, void* scratch, float warm, const float* actions,
+                                      float* obs, float* rew, uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, float* tick_obs,
+                                      float* tick_links, cudaStream_t st) {
+    const int64_t want = (n + MAN_THREADS - 1) / MAN_THREADS;
+    const int full = man_grid(cur_dev());
+    dim3 grid((unsigned)(want < full ? want : full)), block(MAN_THREADS);
+    if (P.cone) snk_man_step_trace_kernel<true><<<grid, block, MAN_RING_BYTES, st>>>(P, state, tgt_scratch, cache, (float4*)scratch, warm, actions, obs, rew, done, ticks, counters, n, tick_obs, tick_links);
+    else snk_man_step_trace_kernel<false><<<grid, block, MAN_RING_BYTES, st>>>(P, state, tgt_scratch, cache, (float4*)scratch, warm, actions, obs, rew, done, ticks, counters, n, tick_obs, tick_links);
+    return cudaGetLastError();
+}
+
+// at most man_grid(dev) CTAs, like the step: the handle's row tables (man_scratch) are indexed by global warp
+cudaError_t snk_man_launch_rollout(const KParams& P, float* state, float* tgt_scratch, float* cache, void* scratch, float warm, const float* weights,
+                                   const float* mean, const float* inv_std, const float* noise, int n_steps, float* returns, float* trace,
+                                   unsigned long long* counters, int64_t n, cudaStream_t st) {
+    RolloutArgs A;
+    A.weights = weights; A.mean = mean; A.inv_std = inv_std; A.noise = noise; A.returns = returns; A.trace = trace; A.n_steps = n_steps;
+    A.queue = nullptr; A.done_steps = nullptr;
+    const int64_t want = (n + MAN_THREADS - 1) / MAN_THREADS;
+    const int full = man_grid(cur_dev());
+    dim3 grid((unsigned)(want < full ? want : full)), block(MAN_THREADS);
+    if (P.cone) snk_man_rollout_kernel<true><<<grid, block, MAN_RING_BYTES, st>>>(P, state, tgt_scratch, cache, (float4*)scratch, warm, A, counters, n);
+    else snk_man_rollout_kernel<false><<<grid, block, MAN_RING_BYTES, st>>>(P, state, tgt_scratch, cache, (float4*)scratch, warm, A, counters, n);
+    return cudaGetLastError();
+}
+
+cudaError_t snk_man_launch_clear(float* cache, const uint8_t* mask, int64_t n, cudaStream_t st) {
+    const int64_t blocks = (n * (MAN_STRIDE / 4) + 255) / 256;
+    snk_man_clear_kernel<<<(unsigned)(blocks < 65536 ? blocks : 65536), 256, 0, st>>>(cache, mask, n);
+    return cudaGetLastError();
+}
+
+cudaError_t snk_man_launch_check(const float* cache, int64_t n, unsigned long long* bad, cudaStream_t st) {
+    const int64_t blocks = (n + 255) / 256;
+    snk_man_check_kernel<<<(unsigned)(blocks < 4096 ? blocks : 4096), 256, 0, st>>>(cache, n, bad);
     return cudaGetLastError();
 }
 

@@ -18,6 +18,7 @@
 // when ITS residual falls below the threshold.  One environment per thread, persistent grid; as in the benchmarked kernel the unit
 // the lanes of a warp share is one physics tick, and a thread whose env-step has ended takes the next environment from a global
 // counter.  Measured and profiled in DESIGN.md section 5 / profiles/README.md (1.1 M env-steps/s at 262 144 environments).
+// The same loop (man_run) also runs the traced step (snk_step_trace) and the fused linear-policy rollout (snk_rollout_linear).
 #pragma once
 #include "snake_exact_core.cuh"
 
@@ -26,6 +27,7 @@
 #define MAN_SLOT_W 8                                     // lp.x lp.y lp.z dist | anchor.x anchor.y impulse_n spare
 #define MAN_CYL_W (MAN_SLOTS * MAN_SLOT_W)               // 32 floats per cylinder
 #define MAN_STRIDE (NC * MAN_CYL_W + NC)                 // floats per environment; the last NC words hold the point counts
+static_assert(MAN_STRIDE == SNK_MAN_STRIDE, "the cache layout of include/snake_b200.h (snk_get_manifold_cache) is this one");
 #define MAN_ROW_V4 5                                     // float4 words per contact point in the scratch table
 #define MAN_WARP_V4 (MAN_NP * MAN_ROW_V4 * 32)           // float4 words per warp of the scratch table
 #define MAN_HULL 32
@@ -522,18 +524,26 @@ __device__ void man_tick(const ExTables& T, const KParams& P, const ManRows& R, 
 }
 
 // -----------------------------------------------------------------------------------------------
-// kernel: one SubprocVecEnv.step() of N environments with persistent manifolds; thread = environment, persistent grid
+// The persistent loop of one thread with persistent manifolds; thread = environment, persistent grid.
+//   TRACE: the mode='test' info stream (snk_step_trace) -- after every tick an environment takes, its observation goes to
+//          tick_obs[env][tick][56] and its link positions to tick_links[env][tick][51] (an aborted tick writes nothing); the
+//          arithmetic is that of the plain step, so obs / rew / done / ticks and the caches are bit-identical to it.
+//   ROLL:  A.n_steps env-steps with a linear policy per environment (snk_rollout_linear): the thread keeps its environment for the
+//          whole rollout and starts the next env-step at once when one ends (policy_targets turns the observation into the next
+//          targets), so no lane waits for its warp; only the return (and the optional policy-input trace) leaves the chip.
+// counters: [0] ticks, [1] PGS sweeps, [2] dones, [3] non-finite resets, [4] next environment to hand out, [7] cached points.
 // -----------------------------------------------------------------------------------------------
 struct ManTgt { // the joint targets of the env-step in flight: the environment's 64 B row of the handle's target scratch array
     float* tg;
     __device__ __forceinline__ float& tgt(int j) const { return tg[j]; }
 };
 
-template <bool CONE>
-__global__ void __launch_bounds__(MAN_THREADS, MAN_MINB)
-snk_man_step_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, float* __restrict__ cache, float4* __restrict__ scratch,
-                    float warm, const float* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done,
-                    int32_t* __restrict__ ticks, unsigned long long* __restrict__ counters, int64_t n) {
+template <bool CONE, bool TRACE, bool ROLL>
+__device__ __forceinline__ void man_run(const KParams& P, float* __restrict__ state, float* __restrict__ tgt_scratch, float* __restrict__ cache,
+                                        float4* __restrict__ scratch, float warm, const float* __restrict__ actions, float* __restrict__ obs,
+                                        float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
+                                        unsigned long long* __restrict__ counters, int64_t n, float* __restrict__ tick_obs,
+                                        float* __restrict__ tick_links, const RolloutArgs& A) {
     const int lane = threadIdx.x & 31;
     const int64_t gw = ((int64_t)blockIdx.x * MAN_THREADS + threadIdx.x) >> 5;
     ManRows R;
@@ -555,6 +565,8 @@ snk_man_step_kernel(const KParams P, float* __restrict__ state, float* __restric
     ExRun run;
     int64_t env = -1;
     bool have = false, first = true;
+    int t = 0;       // ROLL: env-step of the rollout in flight
+    float ret = 0.f; // ROLL: sum of its rewards so far
 #pragma unroll 1
     for (;;) {
         if (!have) {
@@ -565,8 +577,14 @@ snk_man_step_kernel(const KParams P, float* __restrict__ state, float* __restric
             e.st = state + env * SNK_STATE_STRIDE;
             G.tg = tgt_scratch + env * NJ;
             mc = cache + env * MAN_STRIDE;
-            load_targets(P, G, actions + env * P.actdim);
-            ex_load_base(e);
+            if (ROLL) {
+                t = 0;
+                ex_load_base(e);
+                policy_targets(P, G, e, A, env, n, 0);
+            } else {
+                load_targets(P, G, actions + env * P.actdim);
+                ex_load_base(e);
+            }
             ex_step_begin(P, G, e, &run);
         }
         bool fin = !(sqrtf(run.e2) > P.errthr); // checkFeedback (snake.py:228-235); true at once: a zero-tick step (Q5)
@@ -581,20 +599,41 @@ snk_man_step_kernel(const KParams P, float* __restrict__ state, float* __restric
                 run.counter++;
                 run.e2 = to.err2_next;
                 fin = run.counter >= P.maxticks || !(sqrtf(run.e2) > P.errthr);
+                if (TRACE) { // the tick went through: snake.py:291-293
+                    const int64_t row = env * P.maxticks + (run.counter - 1);
+                    if (tick_obs) {
+                        float* to_ = tick_obs + row * SNK_OBS_DIM;
+#pragma unroll 1
+                        for (int k = 0; k < SNK_OBS_DIM; k++) to_[k] = ex_obs_of(e, k);
+                    }
+                    if (tick_links) ex_link_positions(cT, e, tick_links + row * (3 * NB));
+                }
             }
         }
         if (fin) {
             ExStepOut o;
             ex_step_end(cT, P, e, run, &o);
-            rew[env] = o.rew;
-            done[env] = (uint8_t)o.done;
-            if (ticks) ticks[env] = o.ticks;
-            float* go = obs + env * SNK_OBS_DIM;
+            if (ROLL) {
+                c_ticks += (unsigned long long)o.ticks; c_iters += (unsigned long long)o.iters; c_done += o.done; c_bad += o.bad;
+                ret = (t == 0) ? o.rew : ret + o.rew;
+                if (++t < A.n_steps) { // the next env-step of the same environment starts at once, from the observation just made
+                    policy_targets(P, G, e, A, env, n, t);
+                    ex_step_begin(P, G, e, &run);
+                } else {
+                    A.returns[env] = ret;
+                    have = false;
+                }
+            } else {
+                rew[env] = o.rew;
+                done[env] = (uint8_t)o.done;
+                if (ticks) ticks[env] = o.ticks;
+                float* go = obs + env * SNK_OBS_DIM;
 #pragma unroll 1
-            for (int k = 0; k < SNK_OBS_DIM; k += 4)
-                *reinterpret_cast<float4*>(go + k) = make_float4(ex_obs_of(e, k), ex_obs_of(e, k + 1), ex_obs_of(e, k + 2), ex_obs_of(e, k + 3));
-            c_ticks += (unsigned long long)o.ticks; c_iters += (unsigned long long)o.iters; c_done += o.done; c_bad += o.bad;
-            have = false;
+                for (int k = 0; k < SNK_OBS_DIM; k += 4)
+                    *reinterpret_cast<float4*>(go + k) = make_float4(ex_obs_of(e, k), ex_obs_of(e, k + 1), ex_obs_of(e, k + 2), ex_obs_of(e, k + 3));
+                c_ticks += (unsigned long long)o.ticks; c_iters += (unsigned long long)o.iters; c_done += o.done; c_bad += o.bad;
+                have = false;
+            }
         }
     }
     if (c_ticks) atomicAdd(&counters[0], c_ticks);
@@ -602,4 +641,56 @@ snk_man_step_kernel(const KParams P, float* __restrict__ state, float* __restric
     if (c_done) atomicAdd(&counters[2], (unsigned long long)c_done);
     if (c_bad) atomicAdd(&counters[3], (unsigned long long)c_bad);
     if (c_points) atomicAdd(&counters[7], c_points);
+}
+
+// kernel: one SubprocVecEnv.step() of N environments with persistent manifolds
+template <bool CONE>
+__global__ void __launch_bounds__(MAN_THREADS, MAN_MINB)
+snk_man_step_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, float* __restrict__ cache, float4* __restrict__ scratch,
+                    float warm, const float* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done,
+                    int32_t* __restrict__ ticks, unsigned long long* __restrict__ counters, int64_t n) {
+    man_run<CONE, false, false>(P, state, tgt_scratch, cache, scratch, warm, actions, obs, rew, done, ticks, counters, n, nullptr, nullptr, RolloutArgs());
+}
+
+// the same env-step with the mode='test' info stream (snk_step_trace); tick_obs / tick_links: [N][max_ticks][56] / [51], either may be null
+template <bool CONE>
+__global__ void __launch_bounds__(MAN_THREADS, MAN_MINB)
+snk_man_step_trace_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, float* __restrict__ cache, float4* __restrict__ scratch,
+                          float warm, const float* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done,
+                          int32_t* __restrict__ ticks, unsigned long long* __restrict__ counters, int64_t n, float* __restrict__ tick_obs,
+                          float* __restrict__ tick_links) {
+    man_run<CONE, true, false>(P, state, tgt_scratch, cache, scratch, warm, actions, obs, rew, done, ticks, counters, n, tick_obs, tick_links, RolloutArgs());
+}
+
+// A.n_steps env-steps with a linear policy per environment (snk_rollout_linear); A.queue / A.done_steps are not used: a thread keeps its
+// environment, and the threads do not wait for each other, so neither a ready queue nor a cooperative launch is needed
+template <bool CONE>
+__global__ void __launch_bounds__(MAN_THREADS, MAN_MINB)
+snk_man_rollout_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, float* __restrict__ cache, float4* __restrict__ scratch,
+                       float warm, const RolloutArgs A, unsigned long long* __restrict__ counters, int64_t n) {
+    man_run<CONE, false, true>(P, state, tgt_scratch, cache, scratch, warm, nullptr, nullptr, nullptr, nullptr, nullptr, counters, n, nullptr, nullptr, A);
+}
+
+// the cache half of a hard reset (snk_clear_manifold): the MAN_STRIDE floats of every environment whose mask byte is non-zero (all: mask null)
+__global__ void snk_man_clear_kernel(float* __restrict__ cache, const uint8_t* __restrict__ mask, int64_t n) {
+    const int64_t words = n * (MAN_STRIDE / 4), stride = (int64_t)gridDim.x * blockDim.x;
+#pragma unroll 1
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < words; i += stride)
+        if (!mask || mask[i / (MAN_STRIDE / 4)]) reinterpret_cast<float4*>(cache)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
+// input check of snk_set_manifold_cache: *bad += environments of `cache` whose NC count words are not all integers in 0..MAN_SLOTS (a larger
+// count would make pass 1 write more than MAN_NP rows into the next warp's slice of the row table, and pass 2 impulses beyond the slots)
+__global__ void snk_man_check_kernel(const float* __restrict__ cache, int64_t n, unsigned long long* __restrict__ bad) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    unsigned cnt = 0;
+#pragma unroll 1
+    for (int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; env < n; env += stride) {
+        const float* c = cache + env * MAN_STRIDE + NC * MAN_CYL_W;
+        bool ok = true;
+#pragma unroll 1
+        for (int k = 0; k < NC; k++) { const float v = c[k]; ok &= v >= 0.f && v <= (float)MAN_SLOTS && v == truncf(v); } // NaN fails
+        cnt += ok ? 0u : 1u;
+    }
+    if (cnt) atomicAdd(bad, (unsigned long long)cnt);
 }

@@ -27,6 +27,7 @@ from .spaces import Box
 from .urdf_model import OBS_DIM, STATE_STRIDE, NJ, build_model
 
 LINK_POS_DIM = 51  # SNK_LINK_POS_DIM: 17 links x (x, y, z), snake.py:138-146
+MAN_STRIDE = 1056  # SNK_MAN_STRIDE: floats of contact cache per environment (32 cylinders x 4 slots x 8 words + 32 counts)
 
 
 class SnakeVecEnv:
@@ -103,20 +104,23 @@ class SnakeVecEnv:
     def reset(self, mask=None, as_torch=False, hard=False):
         """Soft reset (``snake.py:119-127``) of all environments (or of ``mask``); returns obs [N,56].  ``hard=True`` is
         ``Snake.reset(hardReset=True)`` (``snake.py:88-95``): the world is rebuilt, so the applied-torque / reaction-force
-        slots that a soft reset leaves stale (SURVEY Q9) read zero as well."""
+        slots that a soft reset leaves stale (SURVEY Q9) read zero as well.  With persistent manifolds on, the contact caches of the
+        hard-reset environments are emptied too (a rebuilt world has no cached points; the caches survive SOFT resets only, Q10)."""
         self._check_open()
         torch = self._torch
         if hard:
-            st = self.get_state()
             m = torch.ones(self.num_envs, dtype=torch.bool, device=self.device) if mask is None else \
                 torch.as_tensor(np.asarray(mask) if not torch.is_tensor(mask) else mask, device=self.device).bool()
+            if tuple(m.shape) != (self.num_envs,):
+                raise ValueError("mask must have one entry per environment")
+            st = self.get_state()
             st[m] = 0.0
             st[m, 6] = 1.0  # SNK_S_QUAT + 3
             self.set_state(st)
-            if getattr(self, "_manifold", None):  # a rebuilt world has empty contact caches (they survive SOFT resets only, Q10)
-                if mask is not None and not bool(m.all()):
-                    raise NotImplementedError("hard reset of a subset of the environments while persistent manifolds are on")
-                self.set_manifold(*self._manifold)
+            if getattr(self, "_manifold", None):
+                mb = None if mask is None else m.to(torch.uint8).contiguous()
+                _abi.check(self._lib.snk_clear_manifold(self._h, None if mb is None else self._ptr(mb), self._stream()), self._lib)
+                torch.cuda.current_stream(self.device).synchronize()
         if as_torch or (mask is not None and torch.is_tensor(mask) and mask.is_cuda):
             obs = torch.empty((self.num_envs, OBS_DIM), dtype=torch.float32, device=self.device)
             m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
@@ -284,12 +288,27 @@ class SnakeVecEnv:
 
     def state_dict(self):
         """Checkpoint of the whole batch (the reference never checkpoints simulator state; SURVEY.md section 5):
-        the [N,64] state array on the CPU plus the parameters' bytes."""
-        return {"state": self.get_state().cpu(), "num_envs": self.num_envs, "params": bytes(self.params)}
+        the [N,64] state array on the CPU plus the parameters' bytes.  With persistent manifolds on, also their warm-start
+        factor (``manifold_warm``) and contact caches (``manifold_cache``, [N,1056] on the CPU), so that a restored batch
+        continues bit for bit."""
+        sd = {"state": self.get_state().cpu(), "num_envs": self.num_envs, "params": bytes(self.params)}
+        if getattr(self, "_manifold", None):
+            sd["manifold_warm"] = self._manifold[1]
+            sd["manifold_cache"] = self.get_manifold_cache().cpu()
+        return sd
 
     def load_state_dict(self, sd):
+        """Restore a :meth:`state_dict`.  Raises ``ValueError`` when the checkpoint comes from a batch with another size, other
+        parameters or another contact model (manifolds on / off, another warm-start factor)."""
         if int(sd["num_envs"]) != self.num_envs or bytes(sd["params"]) != bytes(self.params):
             raise ValueError("checkpoint was taken from a batch with another size or other parameters")
+        mine = self._manifold[1] if getattr(self, "_manifold", None) else None
+        theirs = sd.get("manifold_warm")
+        if (mine is None) != (theirs is None) or (mine is not None and float(theirs) != mine):
+            raise ValueError("checkpoint was taken with another contact model (persistent manifolds %s, this batch %s)"
+                             % ("off" if theirs is None else "warm %g" % float(theirs), "off" if mine is None else "warm %g" % mine))
+        if mine is not None:
+            self.set_manifold_cache(sd["manifold_cache"])  # checked before anything is touched
         self.set_state(sd["state"])
 
     def set_manifold(self, on=True, warm=0.1):
@@ -298,6 +317,26 @@ class SnakeVecEnv:
         the oracle's ``Oracle.set_manifold``; the default (off) is the one-point-per-cylinder tick the benchmark runs."""
         _abi.check(self._lib.snk_set_manifold(self._h, int(bool(on)), float(warm)), self._lib)
         self._manifold = (True, float(warm)) if on else None
+
+    def get_manifold_cache(self):
+        """The persistent manifolds' contact caches as a CUDA tensor [N, 1056] (``snk_get_manifold_cache``; layout in
+        include/snake_b200.h at SNK_MAN_STRIDE)."""
+        self._check_open()
+        torch = self._torch
+        c = torch.empty((self.num_envs, MAN_STRIDE), dtype=torch.float32, device=self.device)
+        _abi.check(self._lib.snk_get_manifold_cache(self._h, self._ptr(c), self._stream()), self._lib)
+        return c
+
+    def set_manifold_cache(self, cache):
+        """Load contact caches [N, 1056] (``snk_set_manifold_cache``).  Raises when a point count is not an integer in 0..4; the
+        caches are then left as they were."""
+        self._check_open()
+        torch = self._torch
+        c = torch.as_tensor(cache, dtype=torch.float32, device=self.device).contiguous()
+        if tuple(c.shape) != (self.num_envs, MAN_STRIDE):
+            raise ValueError("manifold cache must be [%d, %d]" % (self.num_envs, MAN_STRIDE))
+        _abi.check(self._lib.snk_set_manifold_cache(self._h, self._ptr(c), self._stream()), self._lib)
+        torch.cuda.current_stream(self.device).synchronize()
 
     def manifold_stats(self):
         """(cached contact points summed over the ticks of the last step launch, ticks) -- ``snk_manifold_stats``."""

@@ -195,7 +195,8 @@ int snk_step_trace(snk_handle* h, const float* actions_dev, float* obs_dev, floa
  * vector wrapper feeds back, ars/train.py:99-110).  weights_dev [N, act_dim, 56]; mean_dev / inv_std_dev [56] or
  * NULL (identity); noise_dev [n_steps, N, 56] or NULL; returns_dev [N] receives the sum of the n_steps rewards;
  * obs_trace_dev [n_steps, N, 56] or NULL receives every x the policy saw (for the caller's running statistics).
- * Only with the exact motor solver (the reference configuration).  State persists as after n_steps snk_step calls. */
+ * Only with the exact motor solver (the reference configuration).  State persists as after n_steps snk_step calls.  With persistent
+ * manifolds on (snk_set_manifold) the manifold kernel runs the rollout, caches included. */
 int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mean_dev, const float* inv_std_dev,
                        const float* noise_dev, int32_t n_steps, float* returns_dev, float* obs_trace_dev, void* stream);
 
@@ -205,9 +206,27 @@ int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mea
  * 4-slot contact cache with Bullet's add / replace / refresh / breaking rules (up to 128 contact points per environment), and
  * the cached normal impulses x warm_start (Bullet: 0.1; 0 = off) start the solver.  The call (re)allocates and CLEARS the caches
  * (4 224 B per environment + 388 MB of row tables per device); they survive soft resets like Bullet's (Q10).  on == 0 returns to
- * the default one-point-per-cylinder tick (deviation D1) and frees the memory.  Only with the exact motor solver; snk_step_trace,
- * snk_tick and snk_rollout_linear are refused while it is on.  Synchronises the device. */
+ * the default one-point-per-cylinder tick (deviation D1) and frees the memory.  Only with the exact motor solver.  While it is on,
+ * snk_step, snk_step_host*, snk_step_trace and snk_rollout_linear run the manifold kernels; snk_tick is refused.  Synchronises the
+ * device. */
 int snk_set_manifold(snk_handle* h, int on, double warm_start);
+
+/* The contact caches of the persistent manifolds: SNK_MAN_STRIDE floats per environment, [N][SNK_MAN_STRIDE].  Cylinder c (0..31)
+ * owns the floats [32 c, 32 c + 32): 4 slots of 8 words, slot s at 32 c + 8 s = (body-frame point x, y, z, distance to the ground
+ * plane, world anchor x, y, normal impulse of the last tick, 0).  Float 1024 + c holds the number of occupied slots of cylinder c, an
+ * integer 0..4 stored as a float; slots at and beyond it are unused.  The caches are simulator state: a checkpoint that should resume
+ * bit for bit needs them next to snk_get_state. */
+#define SNK_MAN_STRIDE 1056
+/* Copy the caches out to cache_dev [N][SNK_MAN_STRIDE] (device memory).  Asynchronous on `stream`, capturable.  SNK_E_ARG when
+ * persistent manifolds are off. */
+int snk_get_manifold_cache(snk_handle* h, float* cache_dev, void* stream);
+/* Copy cache_dev [N][SNK_MAN_STRIDE] (device memory) into the caches.  The count words are checked first (a kernel, then a
+ * synchronisation of `stream`): if any of them is not an integer in 0..4, SNK_E_ARG is returned and the caches are left untouched.
+ * SNK_E_ARG when persistent manifolds are off. */
+int snk_set_manifold_cache(snk_handle* h, const float* cache_dev, void* stream);
+/* Empty the caches of the environments whose mask byte is non-zero (all when mask_dev is NULL): the contact half of a hard reset
+ * (a rebuilt world has no cached points).  Asynchronous on `stream`, capturable.  SNK_E_ARG when persistent manifolds are off. */
+int snk_clear_manifold(snk_handle* h, const uint8_t* mask_dev, void* stream);
 /* out[0] = cached contact points summed over the physics ticks of the last step launch, out[1] = those ticks (their ratio is the
  * mean number of contact rows-triples per tick; the oracle's row_stats).  Synchronises the device. */
 int snk_manifold_stats(snk_handle* h, int64_t out[2]);

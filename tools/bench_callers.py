@@ -139,6 +139,8 @@ def ars(args):
     W = torch.zeros((8, 56), device=dev)
     Wenv = torch.cat([W + 0.03 * delta, W - 0.03 * delta])       # ars/train.py:208-219, v = 0.03
     env = SnakeVecEnv(num_envs=n, device=local)
+    if args.manifold is not None:  # Bullet's persistent contact manifolds + warm starting (snk_set_manifold)
+        env.set_manifold(True, args.manifold)
     T = 50                                                          # ars/train.py:87
     obs = torch.empty((n, 56), device=dev); rew = torch.empty((n,), device=dev); done = torch.empty((n,), dtype=torch.uint8, device=dev)
     cnt = torch.zeros((), device=dev, dtype=torch.float64); mean = torch.zeros(56, device=dev, dtype=torch.float64); m2 = torch.zeros(56, device=dev, dtype=torch.float64)
@@ -197,7 +199,8 @@ def ars(args):
     ms = float(t.item())
     if rank == 0:
         print(json.dumps({"workload": "ARS perturbation sweep, linear policy per environment, all-gather of returns" +
-                          (", fused rollout kernel (snk_rollout_linear)" if args.fused else ", one env.step per step + policy in torch"), "envs_total": n * world,
+                          (", fused rollout kernel (snk_rollout_linear)" if args.fused else ", one env.step per step + policy in torch") +
+                          (", persistent contact manifolds, warm start %g" % args.manifold if args.manifold is not None else ""), "envs_total": n * world,
                           "directions": ndir * world, "steps_per_rollout": T, "rollouts": args.rollouts, "n_gpus": world,
                           "env_steps_per_s": n * world * T * args.rollouts / (ms * 1e-3), "ms_per_sweep": ms / args.rollouts,
                           "returns_gathered": int(full.numel()), "mean_return": float(full.mean()), "welford_count": float(stats[0]),
@@ -214,6 +217,8 @@ if __name__ == "__main__":
     ap.add_argument("--envs-per-gpu", type=int, default=32768)
     ap.add_argument("--rollouts", type=int, default=3)
     ap.add_argument("--fused", action="store_true", help="ars: run every rollout as one snk_rollout_linear launch")
+    ap.add_argument("--manifold", type=float, default=None, metavar="WARM",
+                    help="ars: persistent contact manifolds with warm-start factor WARM (env.set_manifold(True, WARM))")
     ap.add_argument("--graph", action="store_true", help="ppo: capture the whole rollout as one CUDA graph")
     ap.add_argument("--tf32", action="store_true", help="ppo: TF32 tensor-core matmuls in the policy")
     ap.add_argument("--no-validate", action="store_true", help="ppo: torch.distributions argument validation off (no per-step synchronisation)")
