@@ -32,7 +32,6 @@ const char* snk_exact_variant();
 cudaError_t snk_exact_launch_step(const KParams& P, float* state, float* tgt_scratch, const float* actions, float* obs, float* rew, uint8_t* done,
                                   int32_t* ticks, unsigned long long* counters, uint8_t* bucket, int32_t* order, int64_t n, cudaStream_t st,
                                   int* launches, int flag_rows, int* split_buf);
-bool snk_exact_row_flags_supported();
 size_t snk_exact_split_buf_bytes();
 cudaError_t snk_exact_launch_rollout(const KParams& P, float* state, float* tgt_scratch, const float* weights, const float* mean, const float* inv_std,
                                      const float* noise, int n_steps, float* returns, float* trace, int32_t* queue, int32_t* done_steps,
@@ -587,11 +586,11 @@ int snk_step_host_f64(snk_handle* h, const double* actions_host, double* obs_hos
     int rc = ensure_staging(h);
     if (rc) return rc;
     wait_device_work(h);
-    if (zero_copy_enabled() && row_flags_enabled() && h->exact && !h->manifold && snk_exact_row_flags_supported())
+    if (zero_copy_enabled() && row_flags_enabled() && h->exact && !h->manifold)
         return step_host_f64_flags(h, actions_host, obs_host, rew_host, done_host, ticks_host);
     const size_t n = (size_t)h->n, ad = (size_t)h->P.actdim;
     cudaStream_t st = h->hstream;
-    // (Kernels without row flags -- Bullet-order rows, persistent manifolds, the ablation layouts.)  The batch goes through in a few chunks of environments, pipelined: while the GPU steps chunk c the host threads narrow the
+    // (Kernels without row flags -- Bullet-order rows, persistent manifolds.)  The batch goes through in a few chunks of environments, pipelined: while the GPU steps chunk c the host threads narrow the
     // actions of chunk c + 1, and while it steps chunk c + 1 they widen the results of chunk c into the caller's arrays -- only the
     // first narrowing and the last widening are not hidden behind the kernel (SNK_HOST_CHUNKS, default 4 from 2^18 environments).
     static int cfg_chunks = -1;

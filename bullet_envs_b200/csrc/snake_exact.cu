@@ -14,8 +14,6 @@
 //                       w and take 256 of its 512 columns each),
 //   7 words per contact in shared memory ([contact][lane] columns, conflict free, 28 KB per warp = 224 KB per CTA),
 //   2 words per contact in registers (64 of the thread's 255; the normal sweep that reads them is fully unrolled).
-// snk_exact_step_kernel<CONE, SW> is the previous layout (4 warps with 16 words in tensor memory + SW warps with the whole
-// record in shared memory, 7 warps per SM), kept for the ablation (SNK_EXACT_ROWS=split).
 // The lock-step unit of a warp is ONE PHYSICS TICK, not one env-step: a lane whose environment has
 // finished its tick loop writes its outputs and takes the next environment from a global counter while
 // the other lanes keep ticking, so the 0..41 spread of tick counts costs no idle lanes.
@@ -39,18 +37,6 @@
 __constant__ ExTables cT;
 
 #define FULL 0xffffffffu
-#define TWARPS 4 // warps with rows in tensor memory (one per TMEM lane quadrant)
-// Warps with rows in shared memory: a template parameter SW of the kernels.  Three (4 x 4 KB + 3 x 68 KB = 220 KB of shared
-// memory, 224 environments in flight per SM) give the highest steady-state throughput but leave only ~28 KB of the SM's
-// 256 KB for L1, which the per-environment state records then miss; two (152 KB, 192 environments, ~92 KB of L1) are faster
-// whenever the batch is only a few waves of the grid.  The launcher picks per call.
-#define SW_MAX 3
-template <int SW>
-struct StepSmemT {
-    RowsTmemAux t[TWARPS];
-    RowsSmemStore s[SW];
-    uint32_t tmem_base;
-};
 
 // joint targets of one environment: checkBound (SnakeGymEnv.py:82-88) + createAction (snake.py:247-269)
 // + scaling (snake.py:223-225)
@@ -417,90 +403,6 @@ __device__ __forceinline__ void run_rollout_warp(const KParams& P, Rows R, float
     }
 }
 
-template <bool CONE, int SW>
-__global__ void __launch_bounds__((TWARPS + SW) * 32, 1)
-snk_exact_rollout_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, const RolloutArgs A,
-                         unsigned long long* __restrict__ counters, int64_t n) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    StepSmemT<SW>& S = *reinterpret_cast<StepSmemT<SW>*>(smem_raw);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (warp == 0) {
-        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(&S.tmem_base);
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(512));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;");
-    const uint32_t tbase = S.tmem_base;
-    const int64_t first_base = ((int64_t)warp * gridDim.x + blockIdx.x) * 32;
-    const int64_t dyn_base = min((int64_t)gridDim.x * (TWARPS + SW) * 32, n);
-    if (warp < TWARPS) {
-        RowsT R;
-        R.taddr = tbase + ((uint32_t)(32 * warp) << 16);
-        R.s = &S.t[warp];
-        R.lane = lane;
-        run_rollout_warp<CONE>(P, R, state, tgt_scratch, A, counters, n, first_base, dyn_base);
-    }
-    else {
-        RowsS R;
-        R.s = &S.s[warp - TWARPS];
-        R.lane = lane;
-        run_rollout_warp<CONE>(P, R, state, tgt_scratch, A, counters, n, first_base, dyn_base);
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(512));
-}
-
-// 6 warps per CTA, one CTA per SM: rows of warps 0-3 in tensor memory, of warps 4-5 in shared memory
-template <bool CONE, int SW>
-__global__ void __launch_bounds__((TWARPS + SW) * 32, 1)
-snk_exact_step_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, const float* __restrict__ actions, float* __restrict__ obs,
-                      float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks, unsigned long long* __restrict__ counters,
-                      const int32_t* __restrict__ order, int64_t n, int active_warps, int spread) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    StepSmemT<SW>& S = *reinterpret_cast<StepSmemT<SW>*>(smem_raw);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (warp == 0) { // the whole tensor memory of the SM: 512 columns x 128 lanes
-        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(&S.tmem_base);
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(512));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;");
-    const uint32_t tbase = S.tmem_base;
-    // first wave (SNK_EXACT_SPREAD): 3 (default) = warp-major, the warps that have a scheduler to themselves first -- with
-    // the longest-first order the longest env-steps of the launch go to the fastest warps; 1 = warp-major in warp-index
-    // order; 0 = CTA-major; 2 = no static wave, everything from the global counter (ablations).
-    // Warps w and w + 4 share scheduler w: with 7 active warps scheduler 3 has a single warp, with 6 schedulers 2 and 3 do;
-    // the warps that have a scheduler to themselves are the fastest and come first
-    int rank = warp;
-    if (spread == 3 && active_warps == 7) rank = (warp == 3) ? 0 : (warp < 3) ? warp + 1 : warp;
-    else if (spread == 3 && active_warps == 6) rank = (warp == 2) ? 0 : (warp == 3) ? 1 : (warp < 2) ? warp + 2 : warp;
-    const int64_t first_base = (spread == 2) ? -1 : (spread ? ((int64_t)rank * gridDim.x + blockIdx.x) * 32 : ((int64_t)blockIdx.x * active_warps + warp) * 32);
-    const int64_t dyn_base = (spread == 2) ? 0 : min((int64_t)gridDim.x * active_warps * 32, n);
-    if (warp >= active_warps) {
-        // ablation switch (SNK_EXACT_WARPS): this warp takes no environments
-    } else if (warp < TWARPS) {
-        RowsT R;
-        R.taddr = tbase + ((uint32_t)(32 * warp) << 16);
-        R.s = &S.t[warp];
-        R.lane = lane;
-        run_warp<CONE>(P, R, state, tgt_scratch, actions, obs, rew, done, ticks, counters, order, n, first_base, dyn_base);
-    }
-    else {
-        RowsS R;
-        R.s = &S.s[warp - TWARPS];
-        R.lane = lane;
-        run_warp<CONE>(P, R, state, tgt_scratch, actions, obs, rew, done, ticks, counters, order, n, first_base, dyn_base);
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(512));
-}
-
 // ---------------------------------------------------------------------------------------------
 // The benchmarked kernel: 8 warps per CTA, one CTA per SM, every warp's rows spread over tensor memory, shared memory
 // and registers (RowsH).  Warps w and w + 4 run on scheduler w and share TMEM lane quadrant w.
@@ -652,69 +554,6 @@ snk_hyb_rollout_kernel(const KParams P, float* __restrict__ state, float* __rest
     hyb_tmem_free(tbase, warp);
 }
 
-// the same loop with every warp's rows in shared memory: one warp per CTA, 3 CTAs per SM
-// (SNK_EXACT_ROWS=smem; kept for the ablation in DESIGN.md section 6)
-template <bool CONE>
-__global__ void __launch_bounds__(EB, 3)
-snk_exact_step_kernel_smem(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, const float* __restrict__ actions, float* __restrict__ obs,
-                           float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
-                           unsigned long long* __restrict__ counters, const int32_t* __restrict__ order, int64_t n) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    RowsS R;
-    R.s = reinterpret_cast<RowsSmemStore*>(smem_raw);
-    R.lane = threadIdx.x;
-    run_warp<CONE>(P, R, state, tgt_scratch, actions, obs, rew, done, ticks, counters, order, n, (int64_t)blockIdx.x * EB, min((int64_t)gridDim.x * EB, n));
-}
-
-// the env-step with the mode='test' info stream (snk_step_trace): an analysis path for a handful of environments,
-// so the plain shared-memory variant carries it and the benchmarked kernel stays untouched
-template <bool CONE>
-__global__ void __launch_bounds__(EB, 3)
-snk_exact_step_trace_kernel(const KParams P, float* __restrict__ state, float* __restrict__ tgt_scratch, const float* __restrict__ actions, float* __restrict__ obs,
-                            float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
-                            unsigned long long* __restrict__ counters, int64_t n, float* __restrict__ tick_obs, float* __restrict__ tick_links) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    RowsS R;
-    R.s = reinterpret_cast<RowsSmemStore*>(smem_raw);
-    R.lane = threadIdx.x;
-    run_warp<CONE, RowsS, true>(P, R, state, tgt_scratch, actions, obs, rew, done, ticks, counters, nullptr, n, (int64_t)blockIdx.x * EB,
-                                min((int64_t)gridDim.x * EB, n), tick_obs, tick_links);
-}
-
-// n_ticks raw ticks with explicit targets[N,16] (gait script): every environment runs the same number of
-// ticks, so the assignment is static (thread = environment); rows in shared memory
-template <bool CONE>
-__global__ void __launch_bounds__(EB, 3)
-snk_exact_tick_kernel(const KParams P, float* __restrict__ state, const float* __restrict__ targets, unsigned long long* __restrict__ counters,
-                      int64_t n, int n_ticks) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    RowsS R;
-    R.s = reinterpret_cast<RowsSmemStore*>(smem_raw);
-    R.lane = threadIdx.x;
-    const int64_t env = (int64_t)blockIdx.x * EB + threadIdx.x;
-    const bool live = env < n;
-    ExEnv e;
-    e.st = state + (live ? env : 0) * SNK_STATE_STRIDE;
-    e.tid = threadIdx.x;
-    R.tg = const_cast<float*>(targets) + (live ? env : 0) * NJ; // the caller's row itself (only read here)
-    ex_load_base(e);
-    int iters = 0;
-#pragma unroll 1
-    for (int t = 0; t < n_ticks; t++) {
-        bool ab;
-        ExTickOut to;
-        ex_tick<CONE>(cT, P, R, e, live, false, &ab, &to);
-        iters += to.iterations;
-    }
-    if (live) {
-        ex_store_base(e);
-        if (counters) {
-            atomicAdd(&counters[0], (unsigned long long)n_ticks);
-            atomicAdd(&counters[1], (unsigned long long)iters);
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------
 // Longest-first hand-out order.  The tick count of an env-step is known before it runs: with the motor
 // rows imposed exactly the joint error shrinks by (1 - kp) per tick, so ticks = ceil(log(thr / |e|) /
@@ -796,16 +635,14 @@ template __global__ void snk_hyb_step_kernel<true, false>(const KParams, float*,
 // ---------------------------------------------------------------------------------------------
 // launch wrappers used by the C-ABI host code (snake_abi.cu)
 // ---------------------------------------------------------------------------------------------
-enum { ROWS_HYBRID = 0, ROWS_SPLIT = 1, ROWS_SMEM = 2 };
 #define MAX_DEVICES 64
 // Process-wide configuration, written under g_mu by snk_exact_configure (i.e. by snk_create) and read by the launchers.
 // The per-device figures are indexed by the CUDA device ordinal; the ablation switches come from the environment once per create.
 static std::mutex g_mu;
-static int g_sms[MAX_DEVICES], g_smem_ctas[MAX_DEVICES];
-static int g_rows = ROWS_HYBRID; // SNK_EXACT_ROWS = split | smem selects one of the older row layouts (ablation)
+static int g_sms[MAX_DEVICES];
 static bool g_no_sort = false;   // SNK_EXACT_ORDER=index disables the longest-first hand-out (ablation)
-static int g_spread = 3;         // SNK_EXACT_SPREAD: first-wave hand-out policy (see the step kernels)
-static int g_active_warps = 0;   // SNK_EXACT_WARPS=1..8 forces the number of working warps per SM (0: chosen per launch)
+static int g_spread = 3;         // SNK_EXACT_SPREAD: first-wave hand-out policy (see snk_hyb_step_kernel; 1 and 3 are both warp-major)
+static int g_active_warps = 0;   // SNK_EXACT_WARPS=1..8 forces the number of working warps per SM (0: all HWARPS)
 static bool g_balance = true;    // SNK_EXACT_BALANCE=0 disables the two-pool (balanced) hand-out (ablation)
 static bool g_split = true;      // SNK_EXACT_SPLIT=0 disables the split hand-out (env-steps run in two parts; the two pools take over)
 static int g_split_frac_q8 = 154; // SNK_EXACT_SPLIT_FRAC (percent; default: chosen per launch): share of an env-step's predicted ticks in its first part
@@ -813,23 +650,10 @@ static bool g_split_frac_forced = false;
 static int g_split_kmax = 4;       // SNK_EXACT_SPLIT_KMAX: split only up to this many whole env-steps per lane (beyond, the two pools do as well or better)
 static int g_split_min_pct = 3;    // SNK_EXACT_SPLIT_MINPCT: ... and only if the idle lanes of the last wave are at least this share of the batch
 
-// working warps per SM for a batch of n environments.  Hybrid rows: always 8.  Split rows: 7 (three shared-memory warps) once the
-// batch is about two waves of the 7-warp grid, else 6 -- a single wave finishes sooner with fewer warps per scheduler.
-static int warps_for(int64_t n, int dev) {
-    if (g_rows == ROWS_HYBRID) return (g_active_warps >= 1 && g_active_warps <= HWARPS) ? g_active_warps : HWARPS;
-    if (g_active_warps >= 1 && g_active_warps <= TWARPS + SW_MAX) return g_active_warps;
-    return (10 * n >= 18LL * g_sms[dev] * (TWARPS + SW_MAX) * 32) ? TWARPS + 3 : TWARPS + 2;
-}
-
 size_t snk_exact_split_buf_bytes() { return (size_t)(SPLIT_CTAS + SPLIT_MAX + SPLIT_MAX * 8) * sizeof(int); }
 
-// ticks[] as per-environment ready flags (HandOut::flag_rows) exist in the benchmarked kernel only
-bool snk_exact_row_flags_supported() { return g_rows == ROWS_HYBRID; }
-
 const char* snk_exact_variant() {
-    return g_rows == ROWS_HYBRID ? "8 warps/SM, rows in TMEM (8 words) + shared memory (7) + registers (2), 256 envs/SM"
-         : g_rows == ROWS_SPLIT  ? "rows in TMEM (4 warps) + shared memory (2 or 3 warps per launch), 192 / 224 envs/SM"
-                                 : "rows in shared memory, 3 x 32 envs/SM";
+    return "8 warps/SM, rows in TMEM (8 words) + shared memory (7) + registers (2), 256 envs/SM";
 }
 
 // The model tables live in one __constant__ symbol per device: all live handles of a process must share one
@@ -854,8 +678,6 @@ cudaError_t snk_exact_configure(const ExTables* host_tables) {
     if (e != cudaSuccess) return e;
     if (dev < 0 || dev >= MAX_DEVICES) return cudaErrorInvalidDevice;
     memcpy(&g_tables, host_tables, sizeof(ExTables));
-    const char* v = getenv("SNK_EXACT_ROWS");
-    g_rows = (v && v[0] == 's' && v[1] == 'p') ? ROWS_SPLIT : (v && v[0] == 's') ? ROWS_SMEM : ROWS_HYBRID;
     const char* so = getenv("SNK_EXACT_ORDER");
     g_no_sort = so && so[0] == 'i';
     const char* sp = getenv("SNK_EXACT_SPREAD");
@@ -880,20 +702,6 @@ cudaError_t snk_exact_configure(const ExTables* host_tables) {
         e = cudaMemcpyToSymbol(cHullS, hs, sizeof hs);
         if (e == cudaSuccess) e = cudaMemcpyToSymbol(cHullC, hcs, sizeof hcs);
     }
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_kernel_smem<true>, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_kernel_smem<false>, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) e = set_smem(snk_exact_tick_kernel<true>, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) e = set_smem(snk_exact_tick_kernel<false>, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_trace_kernel<true>, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_trace_kernel<false>, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_kernel<true, 2>, sizeof(StepSmemT<2>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_kernel<false, 2>, sizeof(StepSmemT<2>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_kernel<true, 3>, sizeof(StepSmemT<3>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_step_kernel<false, 3>, sizeof(StepSmemT<3>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_rollout_kernel<true, 2>, sizeof(StepSmemT<2>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_rollout_kernel<false, 2>, sizeof(StepSmemT<2>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_rollout_kernel<true, 3>, sizeof(StepSmemT<3>));
-    if (e == cudaSuccess) e = set_smem(snk_exact_rollout_kernel<false, 3>, sizeof(StepSmemT<3>));
     if (e == cudaSuccess) e = set_smem(snk_hyb_step_kernel<true, false>, sizeof(StepSmemH));
     if (e == cudaSuccess) e = set_smem(snk_hyb_step_kernel<false, false>, sizeof(StepSmemH));
     if (e == cudaSuccess) e = set_smem(snk_hyb_step_kernel<true, false, true>, sizeof(StepSmemH));
@@ -923,10 +731,7 @@ cudaError_t snk_exact_configure(const ExTables* host_tables) {
             if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     }
     if (e != cudaSuccess) return e;
-    int per_sm = 0;
     e = cudaDeviceGetAttribute(&g_sms[dev], cudaDevAttrMultiProcessorCount, dev);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, snk_exact_step_kernel_smem<true>, EB, sizeof(RowsSmemStore));
-    if (e == cudaSuccess) g_smem_ctas[dev] = g_sms[dev] * (per_sm > 0 ? per_sm : 1);
     if (e == cudaSuccess) g_live_handles++;
     return e;
 }
@@ -939,8 +744,8 @@ cudaError_t snk_exact_launch_step(const KParams& P, float* state, float* tgt_scr
                                   int32_t* ticks, unsigned long long* counters, uint8_t* bucket, int32_t* order, int64_t n, cudaStream_t st,
                                   int* launches, int flag_rows, int* split_buf) {
     const int dev = cur_dev(), sms = g_sms[dev];
-    const int aw = warps_for(n, dev);
-    const int lanes = g_rows == ROWS_SMEM ? g_smem_ctas[dev] * EB : sms * aw * 32;
+    const int aw = g_active_warps ? g_active_warps : HWARPS;
+    const int lanes = sms * aw * 32;
     const int32_t* use_order = nullptr;
     *launches = 1;
     if (bucket && order && n > lanes && !g_no_sort) {
@@ -952,64 +757,48 @@ cudaError_t snk_exact_launch_step(const KParams& P, float* state, float* tgt_scr
         use_order = order;
         *launches = 3;
     }
-    if (g_rows == ROWS_HYBRID) {
-        // a small batch gets one CTA per warp of environments: all SMs before a second warp per SM
-        const int64_t want = g_spread ? (n + EB - 1) / EB : (n + aw * 32 - 1) / (aw * 32);
-        dim3 grid((unsigned)(want < sms ? want : sms)), block(HWARPS * 32);
-        HandOut H;
-        H.n_long = n; H.short_warps = 0; H.flag_rows = flag_rows;
-        H.split_total = 0; H.split_frac_q8 = g_split_frac_q8; H.bucket = bucket; H.split_buf = split_buf;
-        if (use_order && g_balance && g_split && split_buf && aw == HWARPS && (int)grid.x == sms && sms <= SPLIT_CTAS) {
-            // n = k L + r: the r shortest env-steps are run in two parts (SplitCta).  Model (tools/handout_sim.py, 131 072 environments =
-            // 3.46 L): 110.2 warp iterations with the two pools below, 107.0 split, 104.3 ideal.  Measured on B200 (ms per step, split /
-            // two pools): 50 000 envs 12.1 / 14.6, 62 000 13.7 / 15.3, 100 000 21.2 / 22.7, 131 072 27.8 / 29.2, 162 918 34.9 / 35.3,
-            // 200 000 42.4 / 42.1 -- from five whole env-steps per lane on the two pools do as well, and without the 3 % gate the large
-            // batches lose a little (2^20: 214.9 / 214.2), so: k <= 4 and (L - r) / n >= 3 %.
-            const int64_t L = (int64_t)grid.x * aw * 32, k = n / L, r = n - k * L;
-            if (k >= 1 && k <= g_split_kmax && 16 * r >= L && 100 * (L - r) >= g_split_min_pct * n) {
-                H.split_total = (int)r;
-                // share of the first part: with r <= L / 2 one part per lane, about half each (the lanes without a first part start on
-                // the LONGEST whole env-steps, so a little more than half balances: 60 %, measured); with r > L / 2 the L - r other
-                // lanes finish several second parts each, and the parts even out at r / L (+ 10 points for the same reason)
-                if (!g_split_frac_forced) H.split_frac_q8 = 2 * r <= L ? 154 : (int)((r * 256) / L) + 26 > 230 ? 230 : (int)((r * 256) / L) + 26;
-            }
+    // a small batch gets one CTA per warp of environments: all SMs before a second warp per SM
+    const int64_t want = g_spread ? (n + EB - 1) / EB : (n + aw * 32 - 1) / (aw * 32);
+    dim3 grid((unsigned)(want < sms ? want : sms)), block(HWARPS * 32);
+    HandOut H;
+    H.n_long = n; H.short_warps = 0; H.flag_rows = flag_rows;
+    H.split_total = 0; H.split_frac_q8 = g_split_frac_q8; H.bucket = bucket; H.split_buf = split_buf;
+    if (use_order && g_balance && g_split && split_buf && aw == HWARPS && (int)grid.x == sms && sms <= SPLIT_CTAS) {
+        // n = k L + r: the r shortest env-steps are run in two parts (SplitCta).  Model (tools/handout_sim.py, 131 072 environments =
+        // 3.46 L): 110.2 warp iterations with the two pools below, 107.0 split, 104.3 ideal.  Measured on B200 (ms per step, split /
+        // two pools): 50 000 envs 12.1 / 14.6, 62 000 13.7 / 15.3, 100 000 21.2 / 22.7, 131 072 27.8 / 29.2, 162 918 34.9 / 35.3,
+        // 200 000 42.4 / 42.1 -- from five whole env-steps per lane on the two pools do as well, and without the 3 % gate the large
+        // batches lose a little (2^20: 214.9 / 214.2), so: k <= 4 and (L - r) / n >= 3 %.
+        const int64_t L = (int64_t)grid.x * aw * 32, k = n / L, r = n - k * L;
+        if (k >= 1 && k <= g_split_kmax && 16 * r >= L && 100 * (L - r) >= g_split_min_pct * n) {
+            H.split_total = (int)r;
+            // share of the first part: with r <= L / 2 one part per lane, about half each (the lanes without a first part start on
+            // the LONGEST whole env-steps, so a little more than half balances: 60 %, measured); with r > L / 2 the L - r other
+            // lanes finish several second parts each, and the parts even out at r / L (+ 10 points for the same reason)
+            if (!g_split_frac_forced) H.split_frac_q8 = 2 * r <= L ? 154 : (int)((r * 256) / L) + 26 > 230 ? 230 : (int)((r * 256) / L) + 26;
         }
-        if (H.split_total > 0) {
-            cudaError_t me = cudaMemsetAsync(split_buf, 0, (size_t)(SPLIT_CTAS + H.split_total) * sizeof(int), st);
-            if (me != cudaSuccess) return me; // (a memset node, not a kernel: `launches` stays)
-        } else if (use_order && g_balance && (g_spread == 1 || g_spread == 3)) { // n = k L + r: r lanes (whole warps) run k + 1 env-steps, taken from the shortest
-            const int64_t L = (int64_t)grid.x * aw * 32, k = n / L, r = n - k * L;
-            // Worth it when plain longest-first would end on a long, thinly populated last wave: L - r idle lanes for one env-step out
-            // of n / L per lane, i.e. a loss of about (L - r) / n.  Measured on B200 (ms per step, balanced / plain): 100 000 envs
-            // 22.6 / 23.0, 131 072 29.1 / 30.2, 200 000 42.0 / 44.8, 262 144 53.3 / 53.6 -- but 524 288 109.1 / 106.6: over many waves
-            // the lanes drift away from the k / k + 1 split and the pools only disturb the longest-first order, so it is used for
-            // (L - r) / n >= 3 % only.
-            if (k >= 1 && r > 0 && 100 * (L - r) >= 3 * n) {
-                H.short_warps = (int)((r + 31) / 32);
-                const int64_t n_short = H.short_warps * 32LL * (k + 1);
-                H.n_long = n_short < n ? n - n_short : 0;
-            }
-        }
-        // the split hand-out is an instantiation of its own: the plain one, which runs the large batches, carries none of its code
-#define SNK_LAUNCH_HYB(C, SP) snk_hyb_step_kernel<C, false, SP><<<grid, block, sizeof(StepSmemH), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, use_order, n, aw, g_spread, H, nullptr, nullptr)
-        if (H.split_total > 0) { if (P.cone) SNK_LAUNCH_HYB(true, true); else SNK_LAUNCH_HYB(false, true); }
-        else { if (P.cone) SNK_LAUNCH_HYB(true, false); else SNK_LAUNCH_HYB(false, false); }
-#undef SNK_LAUNCH_HYB
-    } else if (g_rows == ROWS_SPLIT) {
-        const int sw = aw > TWARPS + 2 ? 3 : 2;
-        const int per_cta = (TWARPS + sw) * 32, per_cta_active = aw * 32;
-        const int64_t want = (g_spread == 1 || g_spread == 3) ? (n + EB - 1) / EB : (n + per_cta_active - 1) / per_cta_active;
-        dim3 grid((unsigned)(want < sms ? want : sms)), block(per_cta);
-#define SNK_LAUNCH_STEP(C, S) snk_exact_step_kernel<C, S><<<grid, block, sizeof(StepSmemT<S>), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, use_order, n, aw, g_spread)
-        if (sw == 3) { if (P.cone) SNK_LAUNCH_STEP(true, 3); else SNK_LAUNCH_STEP(false, 3); }
-        else { if (P.cone) SNK_LAUNCH_STEP(true, 2); else SNK_LAUNCH_STEP(false, 2); }
-#undef SNK_LAUNCH_STEP
-    } else {
-        const int64_t warps = (n + EB - 1) / EB;
-        dim3 grid((unsigned)(warps < g_smem_ctas[dev] ? warps : g_smem_ctas[dev])), block(EB);
-        if (P.cone) snk_exact_step_kernel_smem<true><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, use_order, n);
-        else snk_exact_step_kernel_smem<false><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, use_order, n);
     }
+    if (H.split_total > 0) {
+        cudaError_t me = cudaMemsetAsync(split_buf, 0, (size_t)(SPLIT_CTAS + H.split_total) * sizeof(int), st);
+        if (me != cudaSuccess) return me; // (a memset node, not a kernel: `launches` stays)
+    } else if (use_order && g_balance && (g_spread == 1 || g_spread == 3)) { // n = k L + r: r lanes (whole warps) run k + 1 env-steps, taken from the shortest
+        const int64_t L = (int64_t)grid.x * aw * 32, k = n / L, r = n - k * L;
+        // Worth it when plain longest-first would end on a long, thinly populated last wave: L - r idle lanes for one env-step out
+        // of n / L per lane, i.e. a loss of about (L - r) / n.  Measured on B200 (ms per step, balanced / plain): 100 000 envs
+        // 22.6 / 23.0, 131 072 29.1 / 30.2, 200 000 42.0 / 44.8, 262 144 53.3 / 53.6 -- but 524 288 109.1 / 106.6: over many waves
+        // the lanes drift away from the k / k + 1 split and the pools only disturb the longest-first order, so it is used for
+        // (L - r) / n >= 3 % only.
+        if (k >= 1 && r > 0 && 100 * (L - r) >= 3 * n) {
+            H.short_warps = (int)((r + 31) / 32);
+            const int64_t n_short = H.short_warps * 32LL * (k + 1);
+            H.n_long = n_short < n ? n - n_short : 0;
+        }
+    }
+    // the split hand-out is an instantiation of its own: the plain one, which runs the large batches, carries none of its code
+#define SNK_LAUNCH_HYB(C, SP) snk_hyb_step_kernel<C, false, SP><<<grid, block, sizeof(StepSmemH), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, use_order, n, aw, g_spread, H, nullptr, nullptr)
+    if (H.split_total > 0) { if (P.cone) SNK_LAUNCH_HYB(true, true); else SNK_LAUNCH_HYB(false, true); }
+    else { if (P.cone) SNK_LAUNCH_HYB(true, false); else SNK_LAUNCH_HYB(false, false); }
+#undef SNK_LAUNCH_HYB
     return cudaGetLastError();
 }
 
@@ -1067,19 +856,14 @@ cudaError_t snk_man_launch_check(const float* cache, int64_t n, unsigned long lo
 
 cudaError_t snk_exact_launch_step_trace(const KParams& P, float* state, float* tgt_scratch, const float* actions, float* obs, float* rew, uint8_t* done,
                                         int32_t* ticks, unsigned long long* counters, int64_t n, float* tick_obs, float* tick_links, cudaStream_t st) {
+    // the benchmarked kernel's TRACE instantiation: same arithmetic, same bits as snk_step
     const int dev = cur_dev();
     const int64_t warps = (n + EB - 1) / EB;
-    if (g_rows == ROWS_HYBRID) { // the benchmarked kernel's TRACE instantiation: same arithmetic, same bits as snk_step
-        dim3 grid((unsigned)(warps < g_sms[dev] ? warps : g_sms[dev])), block(HWARPS * 32);
-        HandOut H;
-        H.n_long = n; H.short_warps = 0; H.flag_rows = 0;
-        if (P.cone) snk_hyb_step_kernel<true, true><<<grid, block, sizeof(StepSmemH), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, nullptr, n, HWARPS, 1, H, tick_obs, tick_links);
-        else snk_hyb_step_kernel<false, true><<<grid, block, sizeof(StepSmemH), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, nullptr, n, HWARPS, 1, H, tick_obs, tick_links);
-        return cudaGetLastError();
-    }
-    dim3 grid((unsigned)(warps < g_smem_ctas[dev] ? warps : g_smem_ctas[dev])), block(EB);
-    if (P.cone) snk_exact_step_trace_kernel<true><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, n, tick_obs, tick_links);
-    else snk_exact_step_trace_kernel<false><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, n, tick_obs, tick_links);
+    dim3 grid((unsigned)(warps < g_sms[dev] ? warps : g_sms[dev])), block(HWARPS * 32);
+    HandOut H;
+    H.n_long = n; H.short_warps = 0; H.flag_rows = 0;
+    if (P.cone) snk_hyb_step_kernel<true, true><<<grid, block, sizeof(StepSmemH), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, nullptr, n, HWARPS, 1, H, tick_obs, tick_links);
+    else snk_hyb_step_kernel<false, true><<<grid, block, sizeof(StepSmemH), st>>>(P, state, tgt_scratch, actions, obs, rew, done, ticks, counters, nullptr, n, HWARPS, 1, H, tick_obs, tick_links);
     return cudaGetLastError();
 }
 
@@ -1097,34 +881,21 @@ cudaError_t snk_exact_launch_rollout(const KParams& P, float* state, float* tgt_
     const int64_t want = (n + EB - 1) / EB;
     KParams Pc = P;
     void* args[] = {(void*)&Pc, (void*)&state, (void*)&tgt_scratch, (void*)&A, (void*)&counters, (void*)&n};
-    if (g_rows == ROWS_HYBRID) {
-        int per_sm = 0;
-        const void* k = P.cone ? (const void*)snk_hyb_rollout_kernel<true> : (const void*)snk_hyb_rollout_kernel<false>;
-        cudaError_t e = P.cone ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, snk_hyb_rollout_kernel<true>, HWARPS * 32, sizeof(StepSmemH))
-                               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, snk_hyb_rollout_kernel<false>, HWARPS * 32, sizeof(StepSmemH));
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorCooperativeLaunchTooLarge;
-        dim3 grid((unsigned)(want < sms ? want : sms)), block(HWARPS * 32);
-        return cudaLaunchCooperativeKernel(k, grid, block, args, sizeof(StepSmemH), st);
-    }
-    const int sw = warps_for(n, dev) > TWARPS + 2 ? 3 : 2;
-    dim3 grid((unsigned)(want < sms ? want : sms)), block((TWARPS + sw) * 32);
-    const void* k = sw == 3 ? (P.cone ? (const void*)snk_exact_rollout_kernel<true, 3> : (const void*)snk_exact_rollout_kernel<false, 3>)
-                            : (P.cone ? (const void*)snk_exact_rollout_kernel<true, 2> : (const void*)snk_exact_rollout_kernel<false, 2>);
-    return cudaLaunchCooperativeKernel(k, grid, block, args, sw == 3 ? sizeof(StepSmemT<3>) : sizeof(StepSmemT<2>), st);
+    int per_sm = 0;
+    const void* k = P.cone ? (const void*)snk_hyb_rollout_kernel<true> : (const void*)snk_hyb_rollout_kernel<false>;
+    cudaError_t e = P.cone ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, snk_hyb_rollout_kernel<true>, HWARPS * 32, sizeof(StepSmemH))
+                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, snk_hyb_rollout_kernel<false>, HWARPS * 32, sizeof(StepSmemH));
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) return cudaErrorCooperativeLaunchTooLarge;
+    dim3 grid((unsigned)(want < sms ? want : sms)), block(HWARPS * 32);
+    return cudaLaunchCooperativeKernel(k, grid, block, args, sizeof(StepSmemH), st);
 }
 
 cudaError_t snk_exact_launch_tick(const KParams& P, float* state, const float* targets, unsigned long long* counters, int64_t n,
                                   int n_ticks, cudaStream_t st) {
-    if (g_rows == ROWS_HYBRID) {
-        dim3 grid((unsigned)((n + HWARPS * 32 - 1) / (HWARPS * 32))), block(HWARPS * 32);
-        if (P.cone) snk_hyb_tick_kernel<true><<<grid, block, sizeof(StepSmemH), st>>>(P, state, targets, counters, n, n_ticks);
-        else snk_hyb_tick_kernel<false><<<grid, block, sizeof(StepSmemH), st>>>(P, state, targets, counters, n, n_ticks);
-        return cudaGetLastError();
-    }
-    dim3 grid((unsigned)((n + EB - 1) / EB)), block(EB);
-    if (P.cone) snk_exact_tick_kernel<true><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, targets, counters, n, n_ticks);
-    else snk_exact_tick_kernel<false><<<grid, block, sizeof(RowsSmemStore), st>>>(P, state, targets, counters, n, n_ticks);
+    dim3 grid((unsigned)((n + HWARPS * 32 - 1) / (HWARPS * 32))), block(HWARPS * 32);
+    if (P.cone) snk_hyb_tick_kernel<true><<<grid, block, sizeof(StepSmemH), st>>>(P, state, targets, counters, n, n_ticks);
+    else snk_hyb_tick_kernel<false><<<grid, block, sizeof(StepSmemH), st>>>(P, state, targets, counters, n, n_ticks);
     return cudaGetLastError();
 }
 

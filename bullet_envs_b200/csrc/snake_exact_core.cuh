@@ -18,7 +18,8 @@
 //
 // Data placement (DESIGN.md section 5): the 13 base-state floats, the chain cursor and the solver's
 // 6-vector live in registers; the contact-row table (32 contacts x 17 words, re-read by every sweep)
-// lives in tensor memory or shared memory behind a row-storage policy (RowsT / RowsS below); joint
+// lives behind a row-storage policy: on the device RowsH below (tensor memory + shared memory +
+// registers), in the CPU emulation RowsS (shared memory); joint
 // angles/velocities/torques stay in the environment's 256 B record of the handle's [N][64] state
 // array (L1 resident while a lane owns the environment); model tables are read from constant memory
 // at warp-uniform addresses.
@@ -26,7 +27,7 @@
 // The tick is WARP CONVERGENT (every lane executes every row-storage access; masked lanes commit
 // nothing) because the tensor-memory accesses are warp-wide .sync.aligned instructions.
 //
-// Everything except RowsT is __host__ __device__ so that tests/hostemu can run the very same fp32
+// Everything except RowsH is __host__ __device__ so that tests/hostemu can run the very same fp32
 // code on the CPU (development check only; the product library contains the device code only).
 #pragma once
 #include "snake_step.cuh"
@@ -103,21 +104,17 @@ struct ExTables {
 //                (the impulses sit 2 words after rhs invD so that the two operands of  impulse + rhs invD  come from different
 //                register banks when the 16 words arrive in 16 consecutive registers)
 //   N1           rhs_n invD_n                        (only the normal sweep reads it)
-// Words 0-15 live either in shared memory as [word/4][contact][lane] float4 columns (bank = lane) or in
-// TENSOR MEMORY: TMEM lane = thread, column = 16 * contact + word, moved with tcgen05.ld/st 32x32b
-// (sm_100a; the 512 columns of a warp's TMEM quadrant hold exactly 32 contacts x 16 words).  N1 is always in
-// shared memory (4 KB per warp); the joint targets are in global memory (RowsS/RowsT::tg).
+// RowsS keeps words 0-15 in shared memory as [word/4][contact][lane] float4 columns (bank = lane) and N1 beside them
+// (4 KB per warp); RowsH spreads the same words over tensor memory, shared memory and registers.  The joint targets are
+// in global memory (RowsS/RowsH::tg).
 // -----------------------------------------------------------------------------------------------
 struct RowsSmemStore {  // one warp, rows in shared memory: 69 632 B
     float4 X[4][NC][EB];
     float N1[NC][EB];
 };
-struct RowsTmemAux {    // one warp, rows in tensor memory: the shared-memory part, 4 096 B
-    float N1[NC][EB];
-};
 typedef RowsSmemStore ExSmem;
 
-// Both policies also carry `tg`, the 16 joint targets of the lane's current environment: a 64 B row of the handle's target
+// Every policy also carries `tg`, the 16 joint targets of the lane's current environment: a 64 B row of the handle's target
 // scratch array in global memory (written when the lane takes the environment, L1/L2 resident while it owns it).
 struct RowsS {
     static constexpr bool REGN = false; // invD_n / rhs_n invD_n come from the record, not from registers
@@ -149,63 +146,6 @@ struct RowsS {
 };
 
 #ifdef __CUDACC__
-// Rows in tensor memory.  Every access is a warp-wide .sync.aligned instruction: the code using this policy
-// keeps the warp converged (inactive lanes compute on their stale record and are masked at the commits).
-// Loads are asynchronous: the destination registers may only be read after fence4/fence16, which wait for
-// the load AND tie the registers so that the compiler cannot move a use above the wait.
-struct RowsT {
-    static constexpr bool REGN = false;
-    uint32_t taddr;  // TMEM address of this warp's quadrant: base + (32 * (warp % 4) << 16)
-    RowsTmemAux* s;
-    int lane;
-    float* tg;
-    __device__ __forceinline__ float& tgt(int j) const { return tg[j]; }
-    __device__ __forceinline__ void st_n1(int k, float a) const { s->N1[k][lane] = a; }
-    __device__ __forceinline__ void ld_n(int k, float4& x0, float& n1) const {
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=f"(x0.x), "=f"(x0.y), "=f"(x0.z), "=f"(x0.w) : "r"(taddr + 16u * k) : "memory");
-        n1 = s->N1[k][lane];
-    }
-    __device__ __forceinline__ void st4(uint32_t col, float4 v) const {
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr + col), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-    }
-    __device__ __forceinline__ void st16(int k, float4 x0, float4 x1, float4 x2, float4 x3) const {
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr + 16u * k),
-                     "f"(x0.x), "f"(x0.y), "f"(x0.z), "f"(x0.w), "f"(x1.x), "f"(x1.y), "f"(x1.z), "f"(x1.w), "f"(x2.x), "f"(x2.y), "f"(x2.z), "f"(x2.w),
-                     "f"(x3.x), "f"(x3.y), "f"(x3.z), "f"(x3.w) : "memory");
-    }
-    __device__ __forceinline__ void st12(int k, float4 x0, float4 x1, float4 x2) const { st4(16u * k, x0); st4(16u * k + 4u, x1); st4(16u * k + 8u, x2); }
-    __device__ __forceinline__ void ld16(int k, float4& x0, float4& x1, float4& x2, float4& x3) const {
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                     : "=f"(x0.x), "=f"(x0.y), "=f"(x0.z), "=f"(x0.w), "=f"(x1.x), "=f"(x1.y), "=f"(x1.z), "=f"(x1.w), "=f"(x2.x), "=f"(x2.y), "=f"(x2.z),
-                       "=f"(x2.w), "=f"(x3.x), "=f"(x3.y), "=f"(x3.z), "=f"(x3.w)
-                     : "r"(taddr + 16u * k) : "memory");
-    }
-    __device__ __forceinline__ void st_ln(int k, float v) const {
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" ::"r"(taddr + 16u * k), "f"(v) : "memory");
-    }
-    __device__ __forceinline__ void st_lf(int k, float a, float b) const {
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(taddr + 16u * k + 12u), "f"(a), "f"(b) : "memory");
-    }
-    __device__ __forceinline__ void fence4(float4& x0) const {
-        asm volatile("tcgen05.wait::ld.sync.aligned;" : "+f"(x0.x), "+f"(x0.y), "+f"(x0.z), "+f"(x0.w)::"memory");
-    }
-    __device__ __forceinline__ void fence16(float4& x0, float4& x1, float4& x2, float4& x3) const {
-        asm volatile("tcgen05.wait::ld.sync.aligned;"
-                     : "+f"(x0.x), "+f"(x0.y), "+f"(x0.z), "+f"(x0.w), "+f"(x1.x), "+f"(x1.y), "+f"(x1.z), "+f"(x1.w), "+f"(x2.x), "+f"(x2.y), "+f"(x2.z),
-                       "+f"(x2.w), "+f"(x3.x), "+f"(x3.y), "+f"(x3.z), "+f"(x3.w)::"memory");
-    }
-    __device__ __forceinline__ void fence_st() const { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-    __device__ __forceinline__ void st_tmp(int k, float4 t0, float4 t1, float4 t2) const { st12(k, t0, t1, t2); }
-    __device__ __forceinline__ void ld_tmp(int k, float4& t0, float4& t1, float4& t2) const { float4 t3; ld16(k, t0, t1, t2, t3); }
-    __device__ __forceinline__ void fence_tmp(float4& t0, float4& t1, float4& t2) const {
-        asm volatile("tcgen05.wait::ld.sync.aligned;"
-                     : "+f"(t0.x), "+f"(t0.y), "+f"(t0.z), "+f"(t0.w), "+f"(t1.x), "+f"(t1.y), "+f"(t1.z), "+f"(t1.w), "+f"(t2.x), "+f"(t2.y), "+f"(t2.z), "+f"(t2.w)::"memory");
-    }
-    __device__ __forceinline__ void st_rec(int k, float4 x0, float4 x1, float4 x2, float4 x3, float n1) const { st16(k, x0, x1, x2, x3); st_n1(k, n1); }
-    __device__ __forceinline__ void ld_regn(int, float&, float&) const {}
-    __device__ __forceinline__ void clr_lf(int) const {}
-};
-
 // HYBRID rows (the benchmarked kernel): every warp keeps 8 words of a record in tensor memory, 7 in shared memory and 2 in
 // registers, so that EIGHT warps fit on an SM (two per scheduler; two per TMEM lane quadrant, 256 columns each):
 //   tensor memory, column 8 k + w:  0 ln | 1 r.x | 2 r.y | 3 r.z | 4 la | 5 lb | 6 d1.x | 7 d1.y
@@ -216,6 +156,10 @@ struct RowsT {
 //                                   that loop is fully unrolled).  The rows phase, whose contact index is dynamic, parks the two values
 //                                   in the la / lb words (which start at zero); ld_regn / clr_lf move them into the registers and zero
 //                                   the words in an unrolled prologue of the solver.
+// Every tensor-memory access is a warp-wide .sync.aligned instruction: the code using this policy keeps the warp converged
+// (inactive lanes compute on their stale record and are masked at the commits).  Loads are asynchronous: the destination
+// registers may only be read after fence4/fence16/fence_tmp/fence_regn8, which wait for the load AND tie the registers so
+// that the compiler cannot move a use above the wait.
 struct RowsHybStore { // 896 B per contact: the three loads of a record differ by constant offsets from one running address
     struct { float4 A[EB]; float2 B[EB]; float C[EB]; } c[NC];
 };

@@ -267,7 +267,7 @@ int64_t snk_launch_count(const snk_handle* h);
 
 const char* snk_last_error(void);
 const char* snk_build_info(void);
-/* Row layout / warp configuration of the env-step kernel the library currently launches (set at snk_create from SNK_EXACT_ROWS). */
+/* Row layout / warp configuration of the thread-per-environment env-step kernel the library launches. */
 const char* snk_kernel_variant(void);
 
 #ifdef __cplusplus

@@ -33,13 +33,6 @@ def test_hybrid_step_kernel_uses_tensor_memory_shared_memory_and_registers(sass)
     assert k.count("LDS.128") >= 3 and k.count("LDS.64") >= 3
 
 
-def test_split_step_kernel_uses_tensor_memory(sass):
-    txt = open(sass).read()
-    assert "snk_exact_step_kernelILb1ELi3EE" in txt and "snk_exact_step_kernelILb1ELi2EE" in txt    # both warp configurations
-    k = [p for p in txt.split("Function : ") if p.startswith("_Z21snk_exact_step_kernelILb1ELi3EE")][0]
-    assert k.count("LDTM.x16") >= 2 and k.count("LDTM.x4") >= 4 and "STTM" in k                     # tcgen05.ld / tcgen05.st
-
-
 def test_bank_conflict_counter_finds_the_solver_loops(sass):
     """tools/sass_bank_conflicts.py on the hybrid kernel: the rolled friction loop (2 pairs per iteration, MUFU of the cone projection,
     tensor-memory loads) is found, and its register-bank conflicts per pair stay below the first version's 17.7 per contact and sweep"""

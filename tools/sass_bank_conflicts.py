@@ -2,7 +2,7 @@
 """Static count of register-bank conflicts in the hot loops of a kernel, from `cuobjdump -sass` output.
 
     cuobjdump -sass bullet_envs_b200/csrc/libsnake_b200.so > /tmp/lib.sass
-    python tools/sass_bank_conflicts.py /tmp/lib.sass snk_exact_step_kernelILb1ELi3EE
+    python tools/sass_bank_conflicts.py /tmp/lib.sass snk_hyb_step_kernelILb1ELb0ELb0EE
 
 For every backward-branch loop of 80..300 instructions with at least 40 fp32 multiplies it prints
 (kind, instructions, conflicts, .reuse operands, fp instructions): kind = T/S (tensor-memory / shared-memory rows) + F/N (friction /
