@@ -110,6 +110,7 @@ def load_library():
     lib.snk_tick.argtypes = [vp, vp, i32, vp]
     lib.snk_rollout_linear.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp, vp]
     lib.snk_set_manifold.argtypes = [vp, ctypes.c_int, ctypes.c_double]
+    lib.snk_set_bullet_tick.argtypes = [vp, ctypes.c_int, ctypes.c_double]
     lib.snk_manifold_stats.argtypes = [vp, P(i64)]
     lib.snk_get_manifold_cache.argtypes = [vp, vp, vp]
     lib.snk_set_manifold_cache.argtypes = [vp, vp, vp]

@@ -25,6 +25,12 @@ cudaError_t snk_pgs_launch_step(const DevTables* T, const KParams& P, float* sta
                                 float* tick_links = nullptr);
 cudaError_t snk_pgs_launch_tick(const DevTables* T, const KParams& P, float* state, const float* targets, unsigned long long* counters, int64_t n,
                                 int n_ticks, cudaStream_t st);
+// Bullet's literal tick: the warp-per-env kernel on the persistent manifolds' contact set (snake_pgs_manifold.cuh, compiled into snake_pgs.cu)
+cudaError_t snk_bt_configure();
+cudaError_t snk_bt_launch_step(const DevTables* T, const KParams& P, float* state, float* cache, float warm, const float* actions, float* obs, float* rew,
+                               uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs, float* tick_links);
+cudaError_t snk_bt_launch_tick(const DevTables* T, const KParams& P, float* state, float* cache, float warm, const float* targets,
+                               unsigned long long* counters, int64_t n, int n_ticks, cudaStream_t st);
 // thread-per-env kernel with the motor rows eliminated (snake_exact.cu)
 cudaError_t snk_exact_configure(const ExTables* host_tables);
 void snk_exact_release();
@@ -96,6 +102,8 @@ struct snk_handle {
     void* man_scratch;            // device, snk_man_scratch_bytes()
     unsigned long long* man_bad;  // device, 1 word: result of the count-word check of snk_set_manifold_cache
     float man_warm;
+    // Bullet's literal tick (snk_set_bullet_tick): the same caches (man_cache, man_bad, man_warm), no row tables
+    bool bullet;
     // staging for the *_host entry points (allocated on first use)
     cudaEvent_t ev_dev;           // recorded after every state-touching launch on a caller stream; the *_host entry points
     bool ev_valid;                // make their own stream wait on it (a device-path call may still be in flight)
@@ -137,7 +145,9 @@ static cudaError_t launch_step(snk_handle* h, const float* act, float* obs, floa
                                int64_t cnt = -1, int flag_rows = 0) {
     if (cnt < 0) cnt = h->n;
     int launches = 1;
-    cudaError_t e = h->manifold ? snk_man_launch_step(h->P, h->state + off * SNK_STATE_STRIDE, h->tgt + off * NJ,
+    cudaError_t e = h->bullet ? snk_bt_launch_step(h->T, h->P, h->state + off * SNK_STATE_STRIDE, h->man_cache + off * (int64_t)SNK_MAN_STRIDE, h->man_warm,
+                                                   act, obs, rew, done, ticks, h->counters, cnt, st, nullptr, nullptr)
+                    : h->manifold ? snk_man_launch_step(h->P, h->state + off * SNK_STATE_STRIDE, h->tgt + off * NJ,
                                                       h->man_cache + off * (int64_t)snk_man_cache_floats(), h->man_scratch, h->man_warm, act, obs, rew, done,
                                                       ticks, h->counters, cnt, st)
                     : h->exact ? snk_exact_launch_step(h->P, h->state + off * SNK_STATE_STRIDE, h->tgt + off * NJ, act, obs, rew, done, ticks, h->counters,
@@ -314,7 +324,9 @@ int snk_step_trace(snk_handle* h, const float* actions_dev, float* obs_dev, floa
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaMemsetAsync(h->counters, 0, NCOUNTERS * sizeof(unsigned long long), st));
-    if (h->manifold) CU(snk_man_launch_step_trace(h->P, h->state, h->tgt, h->man_cache, h->man_scratch, h->man_warm, actions_dev, obs_dev, rew_dev, done_dev,
+    if (h->bullet) CU(snk_bt_launch_step(h->T, h->P, h->state, h->man_cache, h->man_warm, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters,
+                                         h->n, st, tick_obs_dev, tick_links_dev));
+    else if (h->manifold) CU(snk_man_launch_step_trace(h->P, h->state, h->tgt, h->man_cache, h->man_scratch, h->man_warm, actions_dev, obs_dev, rew_dev, done_dev,
                                                   ticks_dev, h->counters, h->n, tick_obs_dev, tick_links_dev, st));
     else if (h->exact) CU(snk_exact_launch_step_trace(h->P, h->state, h->tgt, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters, h->n, tick_obs_dev,
                                                  tick_links_dev, st));
@@ -328,6 +340,7 @@ int snk_step_trace(snk_handle* h, const float* actions_dev, float* obs_dev, floa
 int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mean_dev, const float* inv_std_dev, const float* noise_dev,
                        int32_t n_steps, float* returns_dev, float* obs_trace_dev, void* stream) {
     if (!h || !weights_dev || !returns_dev || n_steps < 1) return fail(SNK_E_ARG, "snk_rollout_linear: bad argument%s");
+    if (h->bullet) return fail(SNK_E_ARG, "snk_rollout_linear: not available with Bullet's literal tick (snk_set_bullet_tick); use snk_step%s");
     if (!h->exact) return fail(SNK_E_ARG, "snk_rollout_linear: only with the exact motor solver (motor force = inf, kd = 1)%s");
     if (!aligned16(weights_dev)) return fail(SNK_E_ARG, "snk_rollout_linear: weights must be 16-byte aligned%s");
     CU(cudaSetDevice(h->device));
@@ -359,6 +372,7 @@ int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mea
 
 int snk_set_manifold(snk_handle* h, int on, double warm_start) {
     if (!h) return fail(SNK_E_ARG, "snk_set_manifold: null handle%s");
+    if (h->bullet) return fail(SNK_E_ARG, "snk_set_manifold: Bullet's literal tick is on (snk_set_bullet_tick); switch it off first%s");
     if (on && !h->exact) return fail(SNK_E_ARG, "snk_set_manifold: only with the exact motor solver (motor force = inf, kd = 1)%s");
     if (!(warm_start >= 0.0)) return fail(SNK_E_ARG, "snk_set_manifold: warm_start must be >= 0%s");
     CU(cudaSetDevice(h->device));
@@ -384,9 +398,37 @@ int snk_set_manifold(snk_handle* h, int on, double warm_start) {
     return 0;
 }
 
+int snk_set_bullet_tick(snk_handle* h, int on, double warm_start) {
+    if (!h) return fail(SNK_E_ARG, "snk_set_bullet_tick: null handle%s");
+    if (h->manifold) return fail(SNK_E_ARG, "snk_set_bullet_tick: persistent manifolds of the exact tick are on (snk_set_manifold); switch them off first%s");
+    if (!(warm_start >= 0.0)) return fail(SNK_E_ARG, "snk_set_bullet_tick: warm_start must be >= 0%s");
+    CU(cudaSetDevice(h->device));
+    CU(cudaDeviceSynchronize()); // the caches of a step in flight are about to be cleared or freed
+    if (!on) {
+        cudaFree(h->man_cache); cudaFree(h->man_bad);
+        h->man_cache = nullptr; h->man_bad = nullptr; h->bullet = false;
+        return 0;
+    }
+    CU(snk_bt_configure());
+    const size_t cache_bytes = (size_t)h->n * SNK_MAN_STRIDE * sizeof(float);
+    if (!h->man_cache) {
+        if (cudaMalloc(&h->man_cache, cache_bytes) != cudaSuccess || cudaMalloc(&h->man_bad, sizeof(unsigned long long)) != cudaSuccess) {
+            cudaGetLastError();
+            cudaFree(h->man_cache); cudaFree(h->man_bad);
+            h->man_cache = nullptr; h->man_bad = nullptr; h->bullet = false;
+            return fail(SNK_E_NOMEM, "snk_set_bullet_tick: out of device memory (4 224 B per environment)%s");
+        }
+    }
+    CU(cudaMemset(h->man_cache, 0, cache_bytes)); // empty caches, like a freshly loaded world
+    CU(cudaDeviceSynchronize());
+    h->man_warm = (float)warm_start;
+    h->bullet = true;
+    return 0;
+}
+
 int snk_get_manifold_cache(snk_handle* h, float* cache_dev, void* stream) {
     if (!h || !cache_dev) return fail(SNK_E_ARG, "snk_get_manifold_cache: null pointer%s");
-    if (!h->manifold) return fail(SNK_E_ARG, "snk_get_manifold_cache: persistent manifolds are off (snk_set_manifold)%s");
+    if (!h->manifold && !h->bullet) return fail(SNK_E_ARG, "snk_get_manifold_cache: persistent manifolds are off (snk_set_manifold, snk_set_bullet_tick)%s");
     CU(cudaSetDevice(h->device));
     CU(cudaMemcpyAsync(cache_dev, h->man_cache, (size_t)h->n * SNK_MAN_STRIDE * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     mark_device_work(h, (cudaStream_t)stream);
@@ -395,7 +437,7 @@ int snk_get_manifold_cache(snk_handle* h, float* cache_dev, void* stream) {
 
 int snk_set_manifold_cache(snk_handle* h, const float* cache_dev, void* stream) {
     if (!h || !cache_dev) return fail(SNK_E_ARG, "snk_set_manifold_cache: null pointer%s");
-    if (!h->manifold) return fail(SNK_E_ARG, "snk_set_manifold_cache: persistent manifolds are off (snk_set_manifold)%s");
+    if (!h->manifold && !h->bullet) return fail(SNK_E_ARG, "snk_set_manifold_cache: persistent manifolds are off (snk_set_manifold, snk_set_bullet_tick)%s");
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long bad = 0;
@@ -416,7 +458,7 @@ int snk_set_manifold_cache(snk_handle* h, const float* cache_dev, void* stream) 
 
 int snk_clear_manifold(snk_handle* h, const uint8_t* mask_dev, void* stream) {
     if (!h) return fail(SNK_E_ARG, "snk_clear_manifold: null handle%s");
-    if (!h->manifold) return fail(SNK_E_ARG, "snk_clear_manifold: persistent manifolds are off (snk_set_manifold)%s");
+    if (!h->manifold && !h->bullet) return fail(SNK_E_ARG, "snk_clear_manifold: persistent manifolds are off (snk_set_manifold, snk_set_bullet_tick)%s");
     CU(cudaSetDevice(h->device));
     CU(snk_man_launch_clear(h->man_cache, mask_dev, h->n, (cudaStream_t)stream));
     h->launches++;
@@ -440,7 +482,8 @@ int snk_tick(snk_handle* h, const float* targets_dev, int32_t n_ticks, void* str
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaMemsetAsync(h->counters, 0, NCOUNTERS * sizeof(unsigned long long), st));
-    if (h->exact) CU(snk_exact_launch_tick(h->P, h->state, targets_dev, h->counters, h->n, n_ticks, st));
+    if (h->bullet) CU(snk_bt_launch_tick(h->T, h->P, h->state, h->man_cache, h->man_warm, targets_dev, h->counters, h->n, n_ticks, st));
+    else if (h->exact) CU(snk_exact_launch_tick(h->P, h->state, targets_dev, h->counters, h->n, n_ticks, st));
     else CU(snk_pgs_launch_tick(h->T, h->P, h->state, targets_dev, h->counters, h->n, n_ticks, st));
     h->launches++;
     mark_device_work(h, st);
@@ -586,11 +629,11 @@ int snk_step_host_f64(snk_handle* h, const double* actions_host, double* obs_hos
     int rc = ensure_staging(h);
     if (rc) return rc;
     wait_device_work(h);
-    if (zero_copy_enabled() && row_flags_enabled() && h->exact && !h->manifold)
+    if (zero_copy_enabled() && row_flags_enabled() && h->exact && !h->manifold && !h->bullet)
         return step_host_f64_flags(h, actions_host, obs_host, rew_host, done_host, ticks_host);
     const size_t n = (size_t)h->n, ad = (size_t)h->P.actdim;
     cudaStream_t st = h->hstream;
-    // (Kernels without row flags -- Bullet-order rows, persistent manifolds.)  The batch goes through in a few chunks of environments, pipelined: while the GPU steps chunk c the host threads narrow the
+    // (Kernels without row flags -- Bullet-order rows, persistent manifolds, Bullet's literal tick.)  The batch goes through in a few chunks of environments, pipelined: while the GPU steps chunk c the host threads narrow the
     // actions of chunk c + 1, and while it steps chunk c + 1 they widen the results of chunk c into the caller's arrays -- only the
     // first narrowing and the last widening are not hidden behind the kernel (SNK_HOST_CHUNKS, default 4 from 2^18 environments).
     static int cfg_chunks = -1;
@@ -702,7 +745,7 @@ int snk_last_counters(snk_handle* h, int64_t out[4]) {
 
 int snk_manifold_stats(snk_handle* h, int64_t out[2]) {
     if (!h || !out) return fail(SNK_E_ARG, "snk_manifold_stats: null pointer%s");
-    if (!h->manifold) return fail(SNK_E_ARG, "snk_manifold_stats: persistent manifolds are off (snk_set_manifold)%s");
+    if (!h->manifold && !h->bullet) return fail(SNK_E_ARG, "snk_manifold_stats: persistent manifolds are off (snk_set_manifold, snk_set_bullet_tick)%s");
     CU(cudaSetDevice(h->device));
     unsigned long long tmp[8];
     CU(cudaDeviceSynchronize());

@@ -81,8 +81,9 @@ static_assert((sizeof(WarpMemPgs) * WARPS_PER_CTA + 1024) * CTAS_PER_SM <= 23347
 // f6 on body b (b < 0: none) and/or unit torque impulse at joint jm (0: none).  Runs per lane; every
 // lane walks all 16 joints so the shared-memory reads are warp-uniform broadcasts.
 // ---------------------------------------------------------------------------------------------
-__device__ __noinline__ void impulse_response(const WarpMemPgs& W, const DevTables* __restrict__ T, int b, const float* f6, int jm,
-                                              float* out /* ND, shared or local */) {
+template <class WM>
+__device__ __forceinline__ void impulse_response_body(const WM& W, const DevTables* __restrict__ T, int b, const float* f6, int jm,
+                                                      float* out /* ND, shared or local */) {
     float u[NB];
     float p[6] = {0, 0, 0, 0, 0, 0};
 #pragma unroll
@@ -128,6 +129,11 @@ __device__ __noinline__ void impulse_response(const WarpMemPgs& W, const DevTabl
         a[0] = ac[0] + ax[0] * qdd; a[1] = ac[1] + ax[1] * qdd; a[2] = ac[2] + ax[2] * qdd;
         a[3] = ac[3]; a[4] = ac[4]; a[5] = ac[5];
     }
+}
+
+__device__ __noinline__ void impulse_response(const WarpMemPgs& W, const DevTables* __restrict__ T, int b, const float* f6, int jm,
+                                              float* out /* ND, shared or local */) {
+    impulse_response_body(W, T, b, f6, jm, out);
 }
 
 // 6x6 SPD inverse by Cholesky, all in registers (every lane computes the same thing)
@@ -176,7 +182,10 @@ __device__ void sym6_inverse(const float* A /* shared */, float* Ainv /* registe
 // ---------------------------------------------------------------------------------------------
 // one physics tick (oracle: forward_dynamics + tick).  Returns the PGS iteration count.
 // ---------------------------------------------------------------------------------------------
-__device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParams& P, int lane) {
+// passes 1-3 of the articulated-body algorithm (oracle: forward_dynamics): W.nu = unconstrained generalized velocity; W.U, Dinv, uu,
+// IA0inv are kept for the impulse responses
+template <class WM>
+__device__ __forceinline__ void pgs_dynamics(WM& W, const DevTables* __restrict__ T, const KParams& P, int lane) {
     const float dt = P.dt;
     // ---- pass 1: velocity chain (every lane, registers), lane b keeps v_b ----
     float vcur[6], vm[6];
@@ -382,6 +391,62 @@ __device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParam
     }
     __syncwarp();
 
+}
+
+// velocity update with the solver's dv (lane = DoF), joint feedback (lam_m: lane j's motor impulse), semi-implicit Euler
+template <class WM>
+__device__ __forceinline__ void pgs_finish(WM& W, const DevTables* __restrict__ T, const KParams& P, int lane, float dv, float lam_m) {
+    const float dt = P.dt;
+    const bool dof = lane < ND;
+    // ---- velocity update, joint feedback, semi-implicit Euler ----
+    if (dof) { float x = W.nu[lane] + dv; x = (x > P.maxvel) ? P.maxvel : x; W.nuF[lane] = (x < -P.maxvel) ? -P.maxvel : x; } // NaN passes through
+    __syncwarp();
+    float wnew[3], vnew[3];
+    m3v(W.Rw[0], W.nuF, wnew);
+    m3v(W.Rw[0], W.nuF + 3, vnew);
+    float fz;
+    {
+        float vo[3] = {W.s[SNK_S_VEL], W.s[SNK_S_VEL + 1], W.s[SNK_S_VEL + 2]};
+        float nv = sqrtf(dot3(vo, vo)), f[3], zw[3], fzax[3] = {__ldg(&T->fzax[0]), __ldg(&T->fzax[1]), __ldg(&T->fzax[2])};
+        float rm = __ldg(&T->rootm);
+#pragma unroll
+        for (int k = 0; k < 3; k++) f[k] = rm * P.g[k] - rm * vo[k] * (P.kl + P.kl * nv) - rm * (vnew[k] - vo[k]) * P.inv_dt;
+        m3v(W.Rw[0], fzax, zw);
+        fz = dot3(zw, f);
+    }
+    float qn[4];
+    {
+        float ang = sqrtf(dot3(wnew, wnew)), sc;
+        if (ang < 0.001f) sc = 0.5f * dt - dt * dt * dt * 0.020833333333f * ang * ang;
+        else sc = sinf(0.5f * ang * dt) / ang;
+        float ax[3] = {wnew[0] * sc, wnew[1] * sc, wnew[2] * sc};
+        float cw = cosf(ang * dt * 0.5f);
+        const float* q = W.s + SNK_S_QUAT;
+        float x = cw * q[0] + ax[0] * q[3] + ax[1] * q[2] - ax[2] * q[1];
+        float y = cw * q[1] + ax[1] * q[3] + ax[2] * q[0] - ax[0] * q[2];
+        float z = cw * q[2] + ax[2] * q[3] + ax[0] * q[1] - ax[1] * q[0];
+        float w = cw * q[3] - ax[0] * q[0] - ax[1] * q[1] - ax[2] * q[2];
+        float in = 1.f / sqrtf(x * x + y * y + z * z + w * w);
+        qn[0] = x * in; qn[1] = y * in; qn[2] = z * in; qn[3] = w * in;
+    }
+    __syncwarp(); // all lanes have read the old state
+    if (lane < NJ) {
+        float qd = W.nuF[6 + lane];
+        W.s[SNK_S_TAU + lane] = lam_m * P.inv_dt;
+        W.s[SNK_S_QD + lane] = qd;
+        W.s[SNK_S_Q + lane] += qd * dt;
+    }
+    if (lane == 16) W.s[SNK_S_FZ] = fz;
+    if (lane >= 17 && lane < 20) {
+        int k = lane - 17;
+        W.s[SNK_S_VEL + k] = vnew[k]; W.s[SNK_S_OMEGA + k] = wnew[k]; W.s[SNK_S_POS + k] += vnew[k] * dt;
+    }
+    if (lane >= 20 && lane < 24) W.s[SNK_S_QUAT + lane - 20] = qn[lane - 20];
+    __syncwarp();
+}
+
+__device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParams& P, int lane) {
+    pgs_dynamics(W, T, P, lane);
     // ---- constraint rows ----
     float lam_m = 0.f, lam_n = 0.f; // motor / normal impulses owned by this lane (motor row = joint, normal row = cylinder)
     if (lane < NJ) { // motor row of joint lane+1 (A.4)
@@ -674,51 +739,7 @@ __device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParam
         if (res <= P.resthr || it >= P.iters - 1) break;
     }
 
-    // ---- velocity update, joint feedback, semi-implicit Euler ----
-    if (dof) { float x = W.nu[lane] + dv; x = (x > P.maxvel) ? P.maxvel : x; W.nuF[lane] = (x < -P.maxvel) ? -P.maxvel : x; } // NaN passes through
-    __syncwarp();
-    float wnew[3], vnew[3];
-    m3v(W.Rw[0], W.nuF, wnew);
-    m3v(W.Rw[0], W.nuF + 3, vnew);
-    float fz;
-    {
-        float vo[3] = {W.s[SNK_S_VEL], W.s[SNK_S_VEL + 1], W.s[SNK_S_VEL + 2]};
-        float nv = sqrtf(dot3(vo, vo)), f[3], zw[3], fzax[3] = {__ldg(&T->fzax[0]), __ldg(&T->fzax[1]), __ldg(&T->fzax[2])};
-        float rm = __ldg(&T->rootm);
-#pragma unroll
-        for (int k = 0; k < 3; k++) f[k] = rm * P.g[k] - rm * vo[k] * (P.kl + P.kl * nv) - rm * (vnew[k] - vo[k]) * P.inv_dt;
-        m3v(W.Rw[0], fzax, zw);
-        fz = dot3(zw, f);
-    }
-    float qn[4];
-    {
-        float ang = sqrtf(dot3(wnew, wnew)), sc;
-        if (ang < 0.001f) sc = 0.5f * dt - dt * dt * dt * 0.020833333333f * ang * ang;
-        else sc = sinf(0.5f * ang * dt) / ang;
-        float ax[3] = {wnew[0] * sc, wnew[1] * sc, wnew[2] * sc};
-        float cw = cosf(ang * dt * 0.5f);
-        const float* q = W.s + SNK_S_QUAT;
-        float x = cw * q[0] + ax[0] * q[3] + ax[1] * q[2] - ax[2] * q[1];
-        float y = cw * q[1] + ax[1] * q[3] + ax[2] * q[0] - ax[0] * q[2];
-        float z = cw * q[2] + ax[2] * q[3] + ax[0] * q[1] - ax[1] * q[0];
-        float w = cw * q[3] - ax[0] * q[0] - ax[1] * q[1] - ax[2] * q[2];
-        float in = 1.f / sqrtf(x * x + y * y + z * z + w * w);
-        qn[0] = x * in; qn[1] = y * in; qn[2] = z * in; qn[3] = w * in;
-    }
-    __syncwarp(); // all lanes have read the old state
-    if (lane < NJ) {
-        float qd = W.nuF[6 + lane];
-        W.s[SNK_S_TAU + lane] = lam_m * P.inv_dt;
-        W.s[SNK_S_QD + lane] = qd;
-        W.s[SNK_S_Q + lane] += qd * dt;
-    }
-    if (lane == 16) W.s[SNK_S_FZ] = fz;
-    if (lane >= 17 && lane < 20) {
-        int k = lane - 17;
-        W.s[SNK_S_VEL + k] = vnew[k]; W.s[SNK_S_OMEGA + k] = wnew[k]; W.s[SNK_S_POS + k] += vnew[k] * dt;
-    }
-    if (lane >= 20 && lane < 24) W.s[SNK_S_QUAT + lane - 20] = qn[lane - 20];
-    __syncwarp();
+    pgs_finish(W, T, P, lane, dv, lam_m);
     return it + 1;
 }
 
@@ -905,3 +926,6 @@ cudaError_t snk_launch_reset(const KParams& P, float* state, const uint8_t* mask
     snk_reset_kernel<<<grid, block, 0, st>>>(P, state, mask, obs, n, mode);
     return cudaGetLastError();
 }
+
+// Bullet's literal tick: the same tick on the persistent manifolds' contact set (snk_set_bullet_tick)
+#include "snake_pgs_manifold.cuh"

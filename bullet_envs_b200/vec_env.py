@@ -104,7 +104,8 @@ class SnakeVecEnv:
     def reset(self, mask=None, as_torch=False, hard=False):
         """Soft reset (``snake.py:119-127``) of all environments (or of ``mask``); returns obs [N,56].  ``hard=True`` is
         ``Snake.reset(hardReset=True)`` (``snake.py:88-95``): the world is rebuilt, so the applied-torque / reaction-force
-        slots that a soft reset leaves stale (SURVEY Q9) read zero as well.  With persistent manifolds on, the contact caches of the
+        slots that a soft reset leaves stale (SURVEY Q9) read zero as well.  With persistent manifolds on (``set_manifold`` or
+        ``set_bullet_tick``), the contact caches of the
         hard-reset environments are emptied too (a rebuilt world has no cached points; the caches survive SOFT resets only, Q10)."""
         self._check_open()
         torch = self._torch
@@ -117,7 +118,7 @@ class SnakeVecEnv:
             st[m] = 0.0
             st[m, 6] = 1.0  # SNK_S_QUAT + 3
             self.set_state(st)
-            if getattr(self, "_manifold", None):
+            if getattr(self, "_manifold", None) or getattr(self, "_bullet", None) is not None:
                 mb = None if mask is None else m.to(torch.uint8).contiguous()
                 _abi.check(self._lib.snk_clear_manifold(self._h, None if mb is None else self._ptr(mb), self._stream()), self._lib)
                 torch.cuda.current_stream(self.device).synchronize()
@@ -290,24 +291,35 @@ class SnakeVecEnv:
         """Checkpoint of the whole batch (the reference never checkpoints simulator state; SURVEY.md section 5):
         the [N,64] state array on the CPU plus the parameters' bytes.  With persistent manifolds on, also their warm-start
         factor (``manifold_warm``) and contact caches (``manifold_cache``, [N,1056] on the CPU), so that a restored batch
-        continues bit for bit."""
+        continues bit for bit.  With Bullet's literal tick on, ``bullet_tick_warm`` and the caches (``manifold_cache``)."""
         sd = {"state": self.get_state().cpu(), "num_envs": self.num_envs, "params": bytes(self.params)}
         if getattr(self, "_manifold", None):
             sd["manifold_warm"] = self._manifold[1]
             sd["manifold_cache"] = self.get_manifold_cache().cpu()
+        if getattr(self, "_bullet", None) is not None:
+            sd["bullet_tick_warm"] = self._bullet
+            sd["manifold_cache"] = self.get_manifold_cache().cpu()
         return sd
+
+    def _contact_model(self):
+        if getattr(self, "_bullet", None) is not None:
+            return ("Bullet tick", self._bullet)
+        if getattr(self, "_manifold", None):
+            return ("persistent manifolds", self._manifold[1])
+        return ("default", None)
 
     def load_state_dict(self, sd):
         """Restore a :meth:`state_dict`.  Raises ``ValueError`` when the checkpoint comes from a batch with another size, other
-        parameters or another contact model (manifolds on / off, another warm-start factor)."""
+        parameters or another contact model (default, persistent manifolds, Bullet's literal tick, or another warm-start factor)."""
         if int(sd["num_envs"]) != self.num_envs or bytes(sd["params"]) != bytes(self.params):
             raise ValueError("checkpoint was taken from a batch with another size or other parameters")
-        mine = self._manifold[1] if getattr(self, "_manifold", None) else None
-        theirs = sd.get("manifold_warm")
-        if (mine is None) != (theirs is None) or (mine is not None and float(theirs) != mine):
-            raise ValueError("checkpoint was taken with another contact model (persistent manifolds %s, this batch %s)"
-                             % ("off" if theirs is None else "warm %g" % float(theirs), "off" if mine is None else "warm %g" % mine))
-        if mine is not None:
+        mine = self._contact_model()
+        theirs = ("Bullet tick", float(sd["bullet_tick_warm"])) if "bullet_tick_warm" in sd else \
+            ("persistent manifolds", float(sd["manifold_warm"])) if "manifold_warm" in sd else ("default", None)
+        if mine != theirs:
+            fmt = lambda m: m[0] if m[1] is None else "%s, warm %g" % m
+            raise ValueError("checkpoint was taken with another contact model (%s; this batch: %s)" % (fmt(theirs), fmt(mine)))
+        if mine[1] is not None:
             self.set_manifold_cache(sd["manifold_cache"])  # checked before anything is touched
         self.set_state(sd["state"])
 
@@ -317,6 +329,13 @@ class SnakeVecEnv:
         the oracle's ``Oracle.set_manifold``; the default (off) is the one-point-per-cylinder tick the benchmark runs."""
         _abi.check(self._lib.snk_set_manifold(self._h, int(bool(on)), float(warm)), self._lib)
         self._manifold = (True, float(warm)) if on else None
+
+    def set_bullet_tick(self, on=True, warm=0.1):
+        """Bullet's literal tick (``snk_set_bullet_tick``): Bullet-order motor rows relaxed in the PGS together with the persistent
+        manifolds and warm starting (x ``warm``) -- stepSimulation's own tick, on any handle.  Clears the caches; ``on=False`` returns
+        to the handle's own solver.  Mirrors the oracle twin ``BulletTickOracle.set_bullet_tick`` (tests/); ``rollout_linear`` is refused while it is on."""
+        _abi.check(self._lib.snk_set_bullet_tick(self._h, int(bool(on)), float(warm)), self._lib)
+        self._bullet = float(warm) if on else None
 
     def get_manifold_cache(self):
         """The persistent manifolds' contact caches as a CUDA tensor [N, 1056] (``snk_get_manifold_cache``; layout in

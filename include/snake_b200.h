@@ -211,9 +211,20 @@ int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mea
  * device. */
 int snk_set_manifold(snk_handle* h, int on, double warm_start);
 
+/* Bullet's literal tick: Bullet-order motor rows (relaxed inside the projected Gauss-Seidel, as with motor_solver = 0) together with
+ * the persistent manifolds and warm starting of snk_set_manifold -- the one configuration that is stepSimulation's own tick (DESIGN.md
+ * section 4: deviations D1 and D4 both lifted).  Works on any handle: while it is on the handle's motor_solver is not consulted (the
+ * default parameters have an unlimited motor force, so Bullet-order rows are always admissible).  on != 0 (re)allocates and CLEARS
+ * the caches (4 224 B per environment, layout SNK_MAN_STRIDE below); on == 0 frees them and returns to the handle's own solver.
+ * warm_start: factor of the cached normal impulses that start the solver (Bullet: 0.1; 0 = off; < 0 is refused).  While it is on,
+ * snk_step, snk_step_host*, snk_step_trace and snk_tick run the Bullet-tick kernel, the cache entry points and snk_manifold_stats
+ * work, and snk_rollout_linear is refused.  Refused (SNK_E_ARG) while snk_set_manifold is on, and snk_set_manifold is refused while
+ * this is on.  Synchronises the device. */
+int snk_set_bullet_tick(snk_handle* h, int on, double warm_start);
+
 /* The contact caches of the persistent manifolds: SNK_MAN_STRIDE floats per environment, [N][SNK_MAN_STRIDE].  Cylinder c (0..31)
  * owns the floats [32 c, 32 c + 32): 4 slots of 8 words, slot s at 32 c + 8 s = (body-frame point x, y, z, distance to the ground
- * plane, world anchor x, y, normal impulse of the last tick, 0).  Float 1024 + c holds the number of occupied slots of cylinder c, an
+ * plane, world anchor x, y, normal impulse of the last tick, 0).  The same layout serves snk_set_bullet_tick.  Float 1024 + c holds the number of occupied slots of cylinder c, an
  * integer 0..4 stored as a float; slots at and beyond it are unused.  The caches are simulator state: a checkpoint that should resume
  * bit for bit needs them next to snk_get_state. */
 #define SNK_MAN_STRIDE 1056
