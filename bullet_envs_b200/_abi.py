@@ -112,6 +112,8 @@ def load_library():
     lib.snk_set_manifold.argtypes = [vp, ctypes.c_int, ctypes.c_double]
     lib.snk_set_bullet_tick.argtypes = [vp, ctypes.c_int, ctypes.c_double]
     lib.snk_manifold_stats.argtypes = [vp, P(i64)]
+    lib.snk_set_joint_limits.argtypes = [vp, ctypes.c_int, ctypes.c_double]
+    lib.snk_joint_limit_stats.argtypes = [vp, P(i64)]
     lib.snk_get_manifold_cache.argtypes = [vp, vp, vp]
     lib.snk_set_manifold_cache.argtypes = [vp, vp, vp]
     lib.snk_clear_manifold.argtypes = [vp, vp, vp]

@@ -25,11 +25,20 @@ cudaError_t snk_pgs_launch_step(const DevTables* T, const KParams& P, float* sta
                                 float* tick_links = nullptr);
 cudaError_t snk_pgs_launch_tick(const DevTables* T, const KParams& P, float* state, const float* targets, unsigned long long* counters, int64_t n,
                                 int n_ticks, cudaStream_t st);
-// Bullet's literal tick: the warp-per-env kernel on the persistent manifolds' contact set (snake_pgs_manifold.cuh, compiled into snake_pgs.cu)
+// the same kernel with the joint-limit rows at +-lim_angle (snk_set_joint_limits)
+cudaError_t snk_pgs_lim_configure();
+cudaError_t snk_pgs_lim_launch_step(const DevTables* T, const KParams& P, float lim_angle, float* state, const float* actions, float* obs, float* rew,
+                                    uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs,
+                                    float* tick_links);
+cudaError_t snk_pgs_lim_launch_tick(const DevTables* T, const KParams& P, float lim_angle, float* state, const float* targets,
+                                    unsigned long long* counters, int64_t n, int n_ticks, cudaStream_t st);
+// Bullet's literal tick: the warp-per-env kernel on the persistent manifolds' contact set (snake_pgs_manifold.cuh, compiled into snake_pgs.cu);
+// lim = the joint-limit rows' angle, 0 = off
 cudaError_t snk_bt_configure();
-cudaError_t snk_bt_launch_step(const DevTables* T, const KParams& P, float* state, float* cache, float warm, const float* actions, float* obs, float* rew,
-                               uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs, float* tick_links);
-cudaError_t snk_bt_launch_tick(const DevTables* T, const KParams& P, float* state, float* cache, float warm, const float* targets,
+cudaError_t snk_bt_launch_step(const DevTables* T, const KParams& P, float* state, float* cache, float warm, float lim, const float* actions, float* obs,
+                               float* rew, uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs,
+                               float* tick_links);
+cudaError_t snk_bt_launch_tick(const DevTables* T, const KParams& P, float* state, float* cache, float warm, float lim, const float* targets,
                                unsigned long long* counters, int64_t n, int n_ticks, cudaStream_t st);
 // thread-per-env kernel with the motor rows eliminated (snake_exact.cu)
 cudaError_t snk_exact_configure(const ExTables* host_tables);
@@ -67,7 +76,7 @@ cudaError_t snk_launch_self_clearance(const DevTables* T, const float* state, fl
 // reset / observe (snake_pgs.cu)
 cudaError_t snk_launch_reset(const KParams& P, float* state, const uint8_t* mask, float* obs, int64_t n, int mode, cudaStream_t st);
 
-#define NCOUNTERS (8 + 64) // 8 counters + 2 x 64 32-bit words of the hand-out scheduler (histogram, cursors)
+#define NCOUNTERS (8 + 64 + 1) // 8 counters + 2 x 64 32-bit words of the hand-out scheduler (histogram, cursors) + active limit rows
 
 static thread_local char g_err[512] = "";
 
@@ -94,7 +103,8 @@ struct snk_handle {
     int* split_buf;               // device: claim counters, flags and run words of the split hand-out (exact kernel)
     int32_t* roll_queue;          // device: ready queue of snk_rollout_linear, n * (steps - 1) entries (grown on demand)
     size_t roll_queue_len;
-    unsigned long long* counters; // device [NCOUNTERS]: ticks, sweeps, dones, non-finite, work-queue head
+    unsigned long long* counters; // device [NCOUNTERS]: ticks, sweeps, dones, non-finite, work-queue head, ..., active limit rows
+                                  // [SNK_CTR_LIMIT_ROWS]
     int64_t launches;
     // persistent contact manifolds (snk_set_manifold): per-environment caches, the resident threads' row tables, warm-start factor
     bool manifold;
@@ -104,6 +114,8 @@ struct snk_handle {
     float man_warm;
     // Bullet's literal tick (snk_set_bullet_tick): the same caches (man_cache, man_bad, man_warm), no row tables
     bool bullet;
+    // joint-limit rows of the Bullet-order kernels (snk_set_joint_limits): their angle, 0 = off
+    float lim_angle;
     // staging for the *_host entry points (allocated on first use)
     cudaEvent_t ev_dev;           // recorded after every state-touching launch on a caller stream; the *_host entry points
     bool ev_valid;                // make their own stream wait on it (a device-path call may still be in flight)
@@ -146,12 +158,14 @@ static cudaError_t launch_step(snk_handle* h, const float* act, float* obs, floa
     if (cnt < 0) cnt = h->n;
     int launches = 1;
     cudaError_t e = h->bullet ? snk_bt_launch_step(h->T, h->P, h->state + off * SNK_STATE_STRIDE, h->man_cache + off * (int64_t)SNK_MAN_STRIDE, h->man_warm,
-                                                   act, obs, rew, done, ticks, h->counters, cnt, st, nullptr, nullptr)
+                                                   h->lim_angle, act, obs, rew, done, ticks, h->counters, cnt, st, nullptr, nullptr)
                     : h->manifold ? snk_man_launch_step(h->P, h->state + off * SNK_STATE_STRIDE, h->tgt + off * NJ,
                                                       h->man_cache + off * (int64_t)snk_man_cache_floats(), h->man_scratch, h->man_warm, act, obs, rew, done,
                                                       ticks, h->counters, cnt, st)
                     : h->exact ? snk_exact_launch_step(h->P, h->state + off * SNK_STATE_STRIDE, h->tgt + off * NJ, act, obs, rew, done, ticks, h->counters,
                                                      h->bucket + off, h->order + off, cnt, st, &launches, flag_rows, h->split_buf)
+                    : h->lim_angle > 0.f ? snk_pgs_lim_launch_step(h->T, h->P, h->lim_angle, h->state + off * SNK_STATE_STRIDE, act, obs, rew, done, ticks,
+                                                                   h->counters, cnt, st, nullptr, nullptr)
                              : snk_pgs_launch_step(h->T, h->P, h->state + off * SNK_STATE_STRIDE, act, obs, rew, done, ticks, h->counters, cnt, st);
     h->launches += launches;
     mark_device_work(h, st);
@@ -324,12 +338,14 @@ int snk_step_trace(snk_handle* h, const float* actions_dev, float* obs_dev, floa
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaMemsetAsync(h->counters, 0, NCOUNTERS * sizeof(unsigned long long), st));
-    if (h->bullet) CU(snk_bt_launch_step(h->T, h->P, h->state, h->man_cache, h->man_warm, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters,
-                                         h->n, st, tick_obs_dev, tick_links_dev));
+    if (h->bullet) CU(snk_bt_launch_step(h->T, h->P, h->state, h->man_cache, h->man_warm, h->lim_angle, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev,
+                                         h->counters, h->n, st, tick_obs_dev, tick_links_dev));
     else if (h->manifold) CU(snk_man_launch_step_trace(h->P, h->state, h->tgt, h->man_cache, h->man_scratch, h->man_warm, actions_dev, obs_dev, rew_dev, done_dev,
                                                   ticks_dev, h->counters, h->n, tick_obs_dev, tick_links_dev, st));
     else if (h->exact) CU(snk_exact_launch_step_trace(h->P, h->state, h->tgt, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters, h->n, tick_obs_dev,
                                                  tick_links_dev, st));
+    else if (h->lim_angle > 0.f) CU(snk_pgs_lim_launch_step(h->T, h->P, h->lim_angle, h->state, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters,
+                                                            h->n, st, tick_obs_dev, tick_links_dev));
     else CU(snk_pgs_launch_step(h->T, h->P, h->state, actions_dev, obs_dev, rew_dev, done_dev, ticks_dev, h->counters, h->n, st, tick_obs_dev,
                                 tick_links_dev));
     h->launches++;
@@ -402,6 +418,9 @@ int snk_set_bullet_tick(snk_handle* h, int on, double warm_start) {
     if (!h) return fail(SNK_E_ARG, "snk_set_bullet_tick: null handle%s");
     if (h->manifold) return fail(SNK_E_ARG, "snk_set_bullet_tick: persistent manifolds of the exact tick are on (snk_set_manifold); switch them off first%s");
     if (!(warm_start >= 0.0)) return fail(SNK_E_ARG, "snk_set_bullet_tick: warm_start must be >= 0%s");
+    if (!on && h->exact && h->lim_angle > 0.f)
+        return fail(SNK_E_ARG, "snk_set_bullet_tick: the joint limits are on and this handle's motor solver is the exact one, which has no limit rows; "
+                               "switch the joint limits off first%s");
     CU(cudaSetDevice(h->device));
     CU(cudaDeviceSynchronize()); // the caches of a step in flight are about to be cleared or freed
     if (!on) {
@@ -423,6 +442,20 @@ int snk_set_bullet_tick(snk_handle* h, int on, double warm_start) {
     CU(cudaDeviceSynchronize());
     h->man_warm = (float)warm_start;
     h->bullet = true;
+    return 0;
+}
+
+int snk_set_joint_limits(snk_handle* h, int on, double angle) {
+    if (!h) return fail(SNK_E_ARG, "snk_set_joint_limits: null handle%s");
+    if (!on) { h->lim_angle = 0.f; return 0; }
+    if (!(angle > 0.0) || !isfinite(angle) || !((float)angle > 0.f) || !isfinite((float)angle))
+        return fail(SNK_E_ARG, "snk_set_joint_limits: angle must be a finite number > 0 (radians)%s");
+    if (h->exact && !h->bullet)
+        return fail(SNK_E_ARG, "snk_set_joint_limits: this handle runs the exact motor solver (motor_solver 1, or 2 with force = inf and kd = 1), whose 16 "
+                               "unlimited-force motor equalities admit no limit rows; use motor_solver = 0 or snk_set_bullet_tick%s");
+    CU(cudaSetDevice(h->device));
+    CU(snk_pgs_lim_configure()); // (the Bullet-tick kernels are configured by snk_set_bullet_tick)
+    h->lim_angle = (float)angle;
     return 0;
 }
 
@@ -482,8 +515,9 @@ int snk_tick(snk_handle* h, const float* targets_dev, int32_t n_ticks, void* str
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaMemsetAsync(h->counters, 0, NCOUNTERS * sizeof(unsigned long long), st));
-    if (h->bullet) CU(snk_bt_launch_tick(h->T, h->P, h->state, h->man_cache, h->man_warm, targets_dev, h->counters, h->n, n_ticks, st));
+    if (h->bullet) CU(snk_bt_launch_tick(h->T, h->P, h->state, h->man_cache, h->man_warm, h->lim_angle, targets_dev, h->counters, h->n, n_ticks, st));
     else if (h->exact) CU(snk_exact_launch_tick(h->P, h->state, targets_dev, h->counters, h->n, n_ticks, st));
+    else if (h->lim_angle > 0.f) CU(snk_pgs_lim_launch_tick(h->T, h->P, h->lim_angle, h->state, targets_dev, h->counters, h->n, n_ticks, st));
     else CU(snk_pgs_launch_tick(h->T, h->P, h->state, targets_dev, h->counters, h->n, n_ticks, st));
     h->launches++;
     mark_device_work(h, st);
@@ -655,9 +689,9 @@ int snk_step_host_f64(snk_handle* h, const double* actions_host, double* obs_hos
         if (e <= b) { CU(cudaEventRecord(h->ev_chunk[c], st)); continue; }
         float* ha = h->h_act;
         parallel_chunks((e - b) * ad, [=](size_t i0, size_t i1) { for (size_t i = b * ad + i0; i < b * ad + i1; i++) ha[i] = (float)actions_host[i]; });
-        if (c > 0) { // the hand-out words are per launch ([7] is a statistic of the manifold kernel: it accumulates like [0..3])
+        if (c > 0) { // the hand-out words are per launch ([7] and [SNK_CTR_LIMIT_ROWS] are statistics: they accumulate like [0..3])
             CU(cudaMemsetAsync(h->counters + 4, 0, 3 * sizeof(unsigned long long), st));
-            CU(cudaMemsetAsync(h->counters + 8, 0, (NCOUNTERS - 8) * sizeof(unsigned long long), st));
+            CU(cudaMemsetAsync(h->counters + 8, 0, (SNK_CTR_LIMIT_ROWS - 8) * sizeof(unsigned long long), st));
         }
         if (zc) {
             CU(launch_step(h, h->h_act + b * ad, h->h_obs + b * SNK_OBS_DIM, h->h_rew + b, h->h_done + b, h->h_ticks + b, st, (int64_t)b, (int64_t)(e - b)));
@@ -751,6 +785,18 @@ int snk_manifold_stats(snk_handle* h, int64_t out[2]) {
     CU(cudaDeviceSynchronize());
     CU(cudaMemcpy(tmp, h->counters, sizeof tmp, cudaMemcpyDeviceToHost));
     out[0] = (int64_t)tmp[7]; out[1] = (int64_t)tmp[0];
+    return 0;
+}
+
+int snk_joint_limit_stats(snk_handle* h, int64_t out[2]) {
+    if (!h || !out) return fail(SNK_E_ARG, "snk_joint_limit_stats: null pointer%s");
+    if (!(h->lim_angle > 0.f)) return fail(SNK_E_ARG, "snk_joint_limit_stats: the joint limits are off (snk_set_joint_limits)%s");
+    CU(cudaSetDevice(h->device));
+    unsigned long long ticks = 0, rows = 0;
+    CU(cudaDeviceSynchronize());
+    CU(cudaMemcpy(&ticks, h->counters, sizeof ticks, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&rows, h->counters + SNK_CTR_LIMIT_ROWS, sizeof rows, cudaMemcpyDeviceToHost));
+    out[0] = (int64_t)rows; out[1] = (int64_t)ticks;
     return 0;
 }
 

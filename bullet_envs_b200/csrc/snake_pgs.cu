@@ -445,7 +445,81 @@ __device__ __forceinline__ void pgs_finish(WM& W, const DevTables* __restrict__ 
     __syncwarp();
 }
 
-__device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParams& P, int lane) {
+// ---------------------------------------------------------------------------------------------
+// joint-limit rows (snk_set_joint_limits; oracle: tick with set_joint_limits, btMultiBodyJointLimitConstraint of A.1): two unilateral
+// rows per joint, row 2j = +e_(6+j) at the lower limit (penetration q_j + angle) and row 2j + 1 = -e_(6+j) at the upper one
+// (penetration angle - q_j), set up like contact normals.  Both rows reuse the motor row of their joint: response s B_j, inverse
+// effective mass invD_j, in-block Delassus entry A(r_i, r_k) = s_i s_k B_(j_i)[6 + j_k].
+// ---------------------------------------------------------------------------------------------
+// right-hand sides of joint j's two rows; q = q_j at the start of the tick, nu = its post-ABA velocity, iD = invD_j
+__device__ __forceinline__ void limit_rows_rhs(float q, float nu, float angle, const KParams& P, float iD, float& r_lo, float& r_up) {
+    float pen = q + angle, verr = -nu, perr = 0.f;
+    if (pen > 0.f) verr -= pen * P.inv_dt; else perr = -pen * P.erp2 * P.inv_dt;
+    r_lo = (verr + perr) * iD;
+    pen = angle - q; verr = nu; perr = 0.f;
+    if (pen > 0.f) verr -= pen * P.inv_dt; else perr = -pen * P.erp2 * P.inv_dt;
+    r_up = (verr + perr) * iD;
+}
+
+// One sweep over the 32 limit rows in row order, between the motor block and the normal rows (lambda >= 0, no upper bound).  Lane =
+// joint owns BOTH of its rows: the upper row follows the lower one on the same lane (its w is -(w + A d_lo), A = B_j[6 + j]), and since
+// the two rows differ only in sign, the later joints see their net impulse change d_lo - d_up -- one broadcast shuffle per joint, a
+// 16-step serial chain for 32 rows.  Branch free like the motor block (tick).  B: the motor rows' responses (B[j], j < NJ); dvs / dl: the
+// shared copies of dv and of the block's impulse changes; dv, res: this lane's velocity change (lane = DoF) and residual, updated.
+__device__ __forceinline__ void pgs_limit_block(const float (*B)[ND], float* dvs, float* dl, int lane, float r_lo, float r_up, float iD, float Dg,
+                                                float& lam_lo, float& lam_up, float& dv, float& res) {
+    const bool dof = lane < ND;
+    const int ld = dof ? lane : 0;
+    const int lm = lane & (NJ - 1);
+    float w = dvs[6 + lm], dlo_mine = 0.f, dup_mine = 0.f;
+    float bn = B[0][6 + lm]; // A of the coming step, fetched one step ahead of the chain
+#pragma unroll 4
+    for (int i = 0; i < NJ; i++) {
+        const float a = bn;
+        bn = B[i < NJ - 1 ? i + 1 : i][6 + lm];
+        const float d0 = r_lo - w * iD;            // lower row of joint i
+        const float s0 = lam_lo + d0;
+        const bool n0 = s0 < 0.f;
+        const float slo = n0 ? 0.f : s0, dlo = n0 ? -lam_lo : d0;
+        const float wu = -fmaf(a, dlo, w);         // upper row: J = -e, after the lower row's update
+        const float d1 = r_up - wu * iD;
+        const float s1 = lam_up + d1;
+        const bool n1 = s1 < 0.f;
+        const float sup = n1 ? 0.f : s1, dup = n1 ? -lam_up : d1;
+        const float di = __shfl_sync(FULL, dlo - dup, i);
+        const bool mine = lane == i;
+        lam_lo = mine ? slo : lam_lo; lam_up = mine ? sup : lam_up;
+        dlo_mine = mine ? dlo : dlo_mine; dup_mine = mine ? dup : dup_mine;
+        w = fmaf(a, di, w);
+    }
+    dl[lane] = dlo_mine - dup_mine;
+    __syncwarp();
+    if (dof) { // dv += sum_j B_j (d_2j - d_2j+1)
+#pragma unroll
+        for (int i = 0; i < NJ; i++) dv = fmaf(B[i][ld], dl[i], dv);
+        dvs[lane] = dv;
+    }
+    const float r0 = dlo_mine * Dg, r1 = dup_mine * Dg;
+    res = fmaxf(res, fmaxf(r0 * r0, r1 * r1));
+    __syncwarp();
+}
+
+// limit rows with lambda > 0 at the end of the tick (lanes >= NJ hold none)
+__device__ __forceinline__ unsigned limit_rows_active(float lam_lo, float lam_up) {
+    return __popc(__ballot_sync(FULL, lam_lo > 0.f)) + __popc(__ballot_sync(FULL, lam_up > 0.f));
+}
+
+// the record of the warp-per-env kernel with the joint-limit rows on (snk_lim_env_kernel): the limit angle, and the rows active at the
+// end of the ticks so far
+struct WarpMemPgsLim : WarpMemPgs {
+    float lim_angle;
+    unsigned lim_active;
+};
+static_assert((sizeof(WarpMemPgsLim) * WARPS_PER_CTA + 1024) * CTAS_PER_SM <= 233472, "CTAS_PER_SM CTAs of the limit-row kernel must fit into an SM");
+
+// LIM: with the joint-limit rows at +-lim_angle; *lim_active (shared) accumulates the rows active at the end of the tick
+template <bool LIM>
+__device__ int tick_pgs(WarpMemPgs& W, const DevTables* __restrict__ T, const KParams& P, int lane, float lim_angle, unsigned* lim_active) {
     pgs_dynamics(W, T, P, lane);
     // ---- constraint rows ----
     float lam_m = 0.f, lam_n = 0.f; // motor / normal impulses owned by this lane (motor row = joint, normal row = cylinder)
@@ -602,6 +676,8 @@ __device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParam
     }
     const float maximp = P.maximp, mu = P.mu;
     const bool cone = P.cone != 0;
+    float l_rhs_lo = 0.f, l_rhs_up = 0.f, lam_lo = 0.f, lam_up = 0.f; // limit rows of joint lm (lane = joint)
+    if constexpr (LIM) limit_rows_rhs(W.s[SNK_S_Q + lm], W.nu[6 + lm], lim_angle, P, m_iD, l_rhs_lo, l_rhs_up);
     __syncwarp();
     int it = 0;
 #pragma unroll 1
@@ -639,6 +715,7 @@ __device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParam
             res = fmaxf(res, rr * rr);
             __syncwarp();
         }
+        if constexpr (LIM) pgs_limit_block(W.B, W.dvs, W.dl, lane, l_rhs_lo, l_rhs_up, m_iD, m_Dg, lam_lo, lam_up, dv, res);
         {   // ---- normal rows, lane = contact ----
             float w0 = 0.f, w1 = 0.f;
 #pragma unroll
@@ -738,9 +815,20 @@ __device__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParam
         res = __uint_as_float(__reduce_max_sync(FULL, __float_as_uint(res))); // res >= 0: the bit patterns order like the values
         if (res <= P.resthr || it >= P.iters - 1) break;
     }
+    if constexpr (LIM) {
+        const unsigned na = limit_rows_active(lam_lo, lam_up);
+        if (lane == 0) *lim_active += na;
+    }
 
     pgs_finish(W, T, P, lane, dv, lam_m);
     return it + 1;
+}
+
+__device__ __forceinline__ int tick(WarpMemPgs& W, const DevTables* __restrict__ T, const KParams& P, int lane) {
+    return tick_pgs<false>(W, T, P, lane, 0.f, nullptr);
+}
+__device__ __forceinline__ int tick(WarpMemPgsLim& W, const DevTables* __restrict__ T, const KParams& P, int lane) {
+    return tick_pgs<true>(W, T, P, lane, W.lim_angle, &W.lim_active);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -917,6 +1005,49 @@ cudaError_t snk_pgs_launch_tick(const DevTables* T, const KParams& P, float* sta
                             int n_ticks, cudaStream_t st) {
     dim3 grid((unsigned)((n + WARPS_PER_CTA - 1) / WARPS_PER_CTA)), block(WARPS_PER_CTA * 32);
     snk_env_kernel<WarpMemPgs, true, WARPS_PER_CTA, CTAS_PER_SM><<<grid, block, snk_pgs_smem_bytes(), st>>>(T, P, state, targets, nullptr, nullptr, nullptr, nullptr, counters, n, n_ticks);
+    return cudaGetLastError();
+}
+
+// the same env-step with the joint-limit rows at +-lim_angle (snk_set_joint_limits); counters[SNK_CTR_LIMIT_ROWS] accumulates the rows active at the end
+// of the ticks (snk_joint_limit_stats)
+template <bool RAW>
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, CTAS_PER_SM)
+snk_lim_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
+                   float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
+                   unsigned long long* __restrict__ counters, int64_t n, int n_ticks, float* __restrict__ tick_obs, float* __restrict__ tick_links,
+                   float lim_angle) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t env = (int64_t)blockIdx.x * WARPS_PER_CTA + warp;
+    if (env >= n) return;
+    WarpMemPgsLim& W = reinterpret_cast<WarpMemPgsLim*>(smem_raw)[warp];
+    if (lane == 0) { W.lim_angle = lim_angle; W.lim_active = 0; } // visible behind env_step's first __syncwarp
+    env_step<WarpMemPgsLim, RAW>(W, lane, env, T, P, state, in, obs, rew, done, ticks, counters, n_ticks, tick_obs, tick_links);
+    if (lane == 0 && counters && W.lim_active) atomicAdd(&counters[SNK_CTR_LIMIT_ROWS], (unsigned long long)W.lim_active);
+}
+
+size_t snk_pgs_lim_smem_bytes() { return sizeof(WarpMemPgsLim) * WARPS_PER_CTA; }
+
+cudaError_t snk_pgs_lim_configure() {
+    cudaError_t e = cudaFuncSetAttribute(snk_lim_env_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_pgs_lim_smem_bytes());
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(snk_lim_env_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_pgs_lim_smem_bytes());
+}
+
+cudaError_t snk_pgs_lim_launch_step(const DevTables* T, const KParams& P, float lim_angle, float* state, const float* actions, float* obs, float* rew,
+                                    uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs,
+                                    float* tick_links) {
+    dim3 grid((unsigned)((n + WARPS_PER_CTA - 1) / WARPS_PER_CTA)), block(WARPS_PER_CTA * 32);
+    snk_lim_env_kernel<false><<<grid, block, snk_pgs_lim_smem_bytes(), st>>>(T, P, state, actions, obs, rew, done, ticks, counters, n, 0, tick_obs,
+                                                                             tick_links, lim_angle);
+    return cudaGetLastError();
+}
+
+cudaError_t snk_pgs_lim_launch_tick(const DevTables* T, const KParams& P, float lim_angle, float* state, const float* targets,
+                                    unsigned long long* counters, int64_t n, int n_ticks, cudaStream_t st) {
+    dim3 grid((unsigned)((n + WARPS_PER_CTA - 1) / WARPS_PER_CTA)), block(WARPS_PER_CTA * 32);
+    snk_lim_env_kernel<true><<<grid, block, snk_pgs_lim_smem_bytes(), st>>>(T, P, state, targets, nullptr, nullptr, nullptr, nullptr, counters, n,
+                                                                            n_ticks, nullptr, nullptr, lim_angle);
     return cudaGetLastError();
 }
 

@@ -182,9 +182,12 @@ __device__ __forceinline__ int bt_man_update(const DevTables* __restrict__ T, in
 
 // ---------------------------------------------------------------------------------------------
 // one physics tick (oracle: tick with the bullet switch on).  cache: this environment's SNK_MAN_STRIDE floats.  Returns the PGS
-// iteration count; *np_out = cached points of the tick.
+// iteration count; *np_out = cached points of the tick.  LIM: with the joint-limit rows at +-lim_angle (snake_pgs.cu: pgs_limit_block)
+// after the motor rows; *lim_active accumulates the limit rows active at the end of the tick.
 // ---------------------------------------------------------------------------------------------
-__device__ int tick_bt(WarpMemBt& W, const DevTables* __restrict__ T, const KParams& P, int lane, float* __restrict__ cache, float warm, int* np_out) {
+template <bool LIM>
+__device__ int tick_bt(WarpMemBt& W, const DevTables* __restrict__ T, const KParams& P, int lane, float* __restrict__ cache, float warm, int* np_out,
+                       float lim_angle, unsigned* lim_active) {
     pgs_dynamics(W, T, P, lane);
 
     // ---- manifolds, lane = cylinder; the forward-dynamics workspace is dead from here on and holds the point table ----
@@ -355,6 +358,8 @@ __device__ int tick_bt(WarpMemBt& W, const DevTables* __restrict__ T, const KPar
     const int pa = lane & ~1; // the lane pair (pa, pa + 1) holds the two friction rows of one point
     const float maximp = P.maximp, mu = P.mu;
     const bool cone = P.cone != 0;
+    float l_rhs_lo = 0.f, l_rhs_up = 0.f, lam_lo = 0.f, lam_up = 0.f; // limit rows of joint lm (lane = joint)
+    if constexpr (LIM) limit_rows_rhs(W.s[SNK_S_Q + lm], W.nu[6 + lm], lim_angle, P, m_iD, l_rhs_lo, l_rhs_up);
     __syncwarp();
     int it = 0;
 #pragma unroll 1
@@ -392,6 +397,7 @@ __device__ int tick_bt(WarpMemBt& W, const DevTables* __restrict__ T, const KPar
             res = fmaxf(res, rr * rr);
             __syncwarp();
         }
+        if constexpr (LIM) pgs_limit_block(W.B, W.dvs, W.dl, lane, l_rhs_lo, l_rhs_up, m_iD, m_Dg, lam_lo, lam_up, dv, res);
 #pragma unroll 1
         for (int g = 0; g < nbn; g++) { // ---- normal rows of points 32 g .. 32 g + 31, lane = point ----
             const int row = 32 * g + lane;
@@ -492,6 +498,7 @@ __device__ int tick_bt(WarpMemBt& W, const DevTables* __restrict__ T, const KPar
         res = __uint_as_float(__reduce_max_sync(FULL, __float_as_uint(res))); // res >= 0: the bit patterns order like the values
         if (res <= P.resthr || it >= P.iters - 1) break;
     }
+    if constexpr (LIM) *lim_active += limit_rows_active(lam_lo, lam_up);
     // the normal impulses go back into the slots (m_appliedImpulse), lane = cylinder
 #pragma unroll
     for (int q = 0; q < BT_SLOTS; q++)
@@ -504,19 +511,15 @@ __device__ int tick_bt(WarpMemBt& W, const DevTables* __restrict__ T, const KPar
 // ---------------------------------------------------------------------------------------------
 // kernel: snk_env_kernel's task logic (snake_task.cuh) around tick_bt, one warp (= one CTA) per environment.  RAW = false: one
 // SubprocVecEnv.step (tick_obs / tick_links: the mode='test' info stream, either may be null); RAW = true: n_ticks raw ticks with
-// targets[N,16].  cache: [N][SNK_MAN_STRIDE].  counters[7] accumulates the cached points over the ticks (snk_manifold_stats).
+// targets[N,16].  cache: [N][SNK_MAN_STRIDE].  counters[7] accumulates the cached points over the ticks (snk_manifold_stats); with LIM
+// (the joint-limit rows at +-lim_angle) counters[SNK_CTR_LIMIT_ROWS] the limit rows active at the end of the ticks (snk_joint_limit_stats).
 // ---------------------------------------------------------------------------------------------
-template <bool RAW>
-__global__ void __launch_bounds__(32, BT_CTAS_PER_SM)
-snk_bt_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
-                  float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
-                  unsigned long long* __restrict__ counters, int64_t n, int n_ticks, float* __restrict__ tick_obs, float* __restrict__ tick_links,
-                  float* __restrict__ cache, float warm) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int lane = threadIdx.x & 31;
-    const int64_t env = blockIdx.x;
-    if (env >= n) return;
-    WarpMemBt& W = *reinterpret_cast<WarpMemBt*>(smem_raw);
+template <bool RAW, bool LIM>
+__device__ __forceinline__ void bt_env_step(WarpMemBt& W, int lane, int64_t env, const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
+                                            float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
+                                            unsigned long long* __restrict__ counters, int n_ticks, float* __restrict__ tick_obs,
+                                            float* __restrict__ tick_links, float* __restrict__ cache, float warm, float lim_angle) {
+    unsigned lim_active = 0;
     float* mc = cache + env * SNK_MAN_STRIDE;
     float* gs = state + env * SNK_STATE_STRIDE;
     W.s[lane] = gs[lane];
@@ -545,7 +548,7 @@ snk_bt_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __res
     if (RAW) {
         for (int t = 0; t < n_ticks; t++) {
             int np;
-            iters += tick_bt(W, T, P, lane, mc, warm, &np);
+            iters += tick_bt<LIM>(W, T, P, lane, mc, warm, &np, LIM ? lim_angle : 0.f, LIM ? &lim_active : nullptr);
             points += (unsigned long long)np;
             counter++;
             height = fk(W, T, lane);
@@ -557,7 +560,7 @@ snk_bt_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __res
             for (int j = 0; j < NJ; j++) { float d = W.target[j] - W.s[SNK_S_Q + j]; e2 += d * d; }
             if (!(sqrtf(e2) > P.errthr)) break;
             int np;
-            iters += tick_bt(W, T, P, lane, mc, warm, &np);
+            iters += tick_bt<LIM>(W, T, P, lane, mc, warm, &np, LIM ? lim_angle : 0.f, LIM ? &lim_active : nullptr);
             points += (unsigned long long)np;
             height = fk(W, T, lane);
             if (tick_obs) { // mode='test' info stream (snake.py:291-292): the observation after this tick
@@ -579,6 +582,7 @@ snk_bt_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __res
         }
     }
     if (lane == 0 && counters && points) atomicAdd(&counters[7], points);
+    if constexpr (LIM) { if (lane == 0 && counters && lim_active) atomicAdd(&counters[SNK_CTR_LIMIT_ROWS], (unsigned long long)lim_active); }
     if (RAW) {
         gs[lane] = W.s[lane];
         gs[lane + 32] = W.s[lane + 32];
@@ -618,24 +622,65 @@ snk_bt_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __res
     }
 }
 
+template <bool RAW>
+__global__ void __launch_bounds__(32, BT_CTAS_PER_SM)
+snk_bt_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
+                  float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
+                  unsigned long long* __restrict__ counters, int64_t n, int n_ticks, float* __restrict__ tick_obs, float* __restrict__ tick_links,
+                  float* __restrict__ cache, float warm) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31;
+    const int64_t env = blockIdx.x;
+    if (env >= n) return;
+    WarpMemBt& W = *reinterpret_cast<WarpMemBt*>(smem_raw);
+    bt_env_step<RAW, false>(W, lane, env, T, P, state, in, obs, rew, done, ticks, counters, n_ticks, tick_obs, tick_links, cache, warm, 0.f);
+}
+
+// Bullet's literal tick with the joint-limit rows (snk_set_joint_limits together with snk_set_bullet_tick)
+template <bool RAW>
+__global__ void __launch_bounds__(32, BT_CTAS_PER_SM)
+snk_bt_lim_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
+                      float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
+                      unsigned long long* __restrict__ counters, int64_t n, int n_ticks, float* __restrict__ tick_obs, float* __restrict__ tick_links,
+                      float* __restrict__ cache, float warm, float lim_angle) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31;
+    const int64_t env = blockIdx.x;
+    if (env >= n) return;
+    WarpMemBt& W = *reinterpret_cast<WarpMemBt*>(smem_raw);
+    bt_env_step<RAW, true>(W, lane, env, T, P, state, in, obs, rew, done, ticks, counters, n_ticks, tick_obs, tick_links, cache, warm, lim_angle);
+}
+
 size_t snk_bt_smem_bytes() { return sizeof(WarpMemBt); }
 
 cudaError_t snk_bt_configure() {
     cudaError_t e = cudaFuncSetAttribute(snk_bt_env_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_bt_smem_bytes());
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(snk_bt_env_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_bt_smem_bytes());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(snk_bt_env_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_bt_smem_bytes());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(snk_bt_lim_env_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_bt_smem_bytes());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(snk_bt_lim_env_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snk_bt_smem_bytes());
+    return e;
 }
 
-cudaError_t snk_bt_launch_step(const DevTables* T, const KParams& P, float* state, float* cache, float warm, const float* actions, float* obs, float* rew,
-                               uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs, float* tick_links) {
-    snk_bt_env_kernel<false><<<(unsigned)n, 32, snk_bt_smem_bytes(), st>>>(T, P, state, actions, obs, rew, done, ticks, counters, n, 0, tick_obs, tick_links,
-                                                                           cache, warm);
+// lim: the joint-limit rows' angle, 0 = off (the kernels without them)
+cudaError_t snk_bt_launch_step(const DevTables* T, const KParams& P, float* state, float* cache, float warm, float lim, const float* actions, float* obs,
+                               float* rew, uint8_t* done, int32_t* ticks, unsigned long long* counters, int64_t n, cudaStream_t st, float* tick_obs,
+                               float* tick_links) {
+    if (lim > 0.f)
+        snk_bt_lim_env_kernel<false><<<(unsigned)n, 32, snk_bt_smem_bytes(), st>>>(T, P, state, actions, obs, rew, done, ticks, counters, n, 0, tick_obs,
+                                                                                   tick_links, cache, warm, lim);
+    else
+        snk_bt_env_kernel<false><<<(unsigned)n, 32, snk_bt_smem_bytes(), st>>>(T, P, state, actions, obs, rew, done, ticks, counters, n, 0, tick_obs, tick_links,
+                                                                               cache, warm);
     return cudaGetLastError();
 }
 
-cudaError_t snk_bt_launch_tick(const DevTables* T, const KParams& P, float* state, float* cache, float warm, const float* targets,
+cudaError_t snk_bt_launch_tick(const DevTables* T, const KParams& P, float* state, float* cache, float warm, float lim, const float* targets,
                                unsigned long long* counters, int64_t n, int n_ticks, cudaStream_t st) {
-    snk_bt_env_kernel<true><<<(unsigned)n, 32, snk_bt_smem_bytes(), st>>>(T, P, state, targets, nullptr, nullptr, nullptr, nullptr, counters, n, n_ticks,
-                                                                          nullptr, nullptr, cache, warm);
+    if (lim > 0.f)
+        snk_bt_lim_env_kernel<true><<<(unsigned)n, 32, snk_bt_smem_bytes(), st>>>(T, P, state, targets, nullptr, nullptr, nullptr, nullptr, counters, n,
+                                                                                  n_ticks, nullptr, nullptr, cache, warm, lim);
+    else
+        snk_bt_env_kernel<true><<<(unsigned)n, 32, snk_bt_smem_bytes(), st>>>(T, P, state, targets, nullptr, nullptr, nullptr, nullptr, counters, n, n_ticks,
+                                                                              nullptr, nullptr, cache, warm);
     return cudaGetLastError();
 }

@@ -9,6 +9,9 @@
 #define NC SNK_NC
 #define ND SNK_NDOF
 #define NROW (NJ + 3 * NC)
+// word of the device counters that accumulates the joint-limit rows active at the end of the ticks (snk_joint_limit_stats): behind the
+// 8 statistics / hand-out words and the 64 words of the exact kernel's hand-out scheduler, so that no kernel's word is shared
+#define SNK_CTR_LIMIT_ROWS (8 + 64)
 
 // Model tables in fp32, resident in global memory (read through the read-only path; every
 // access is either warp-uniform or one element per lane, so they live in L1 after first touch).

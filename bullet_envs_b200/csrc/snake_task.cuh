@@ -25,18 +25,14 @@ __device__ __forceinline__ void soft_reset(WM& W, const KParams& P, int lane) { 
     }
 }
 
-// RAW = false: one SubprocVecEnv.step.  RAW = true: n_ticks raw ticks with targets[N,16] (gait script).
-template <class WM, bool RAW, int WARPS, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-snk_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
-                float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
-                unsigned long long* __restrict__ counters, int64_t n, int n_ticks, float* __restrict__ tick_obs = nullptr,
-                float* __restrict__ tick_links = nullptr) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t env = (int64_t)blockIdx.x * WARPS + warp;
-    if (env >= n) return;
-    WM& W = reinterpret_cast<WM*>(smem_raw)[warp];
+// One env-step (or n_ticks raw ticks) of environment env on its warp's record W.  RAW = false: one SubprocVecEnv.step.  RAW = true:
+// n_ticks raw ticks with targets[N,16] (gait script).  P is taken by value like the kernel parameter it is: passed by reference it
+// changes the code generated for the existing kernels.
+template <class WM, bool RAW>
+__device__ __forceinline__ void env_step(WM& W, int lane, int64_t env, const DevTables* __restrict__ T, const KParams P, float* __restrict__ state,
+                                         const float* __restrict__ in, float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done,
+                                         int32_t* __restrict__ ticks, unsigned long long* __restrict__ counters, int n_ticks,
+                                         float* __restrict__ tick_obs, float* __restrict__ tick_links) {
     float* gs = state + env * SNK_STATE_STRIDE;
     W.s[lane] = gs[lane];
     W.s[lane + 32] = gs[lane + 32];
@@ -129,5 +125,19 @@ snk_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restri
             if (bad) atomicAdd(&counters[3], 1ull);
         }
     }
+}
+
+template <class WM, bool RAW, int WARPS, int MINB>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+snk_env_kernel(const DevTables* __restrict__ T, const KParams P, float* __restrict__ state, const float* __restrict__ in,
+                float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done, int32_t* __restrict__ ticks,
+                unsigned long long* __restrict__ counters, int64_t n, int n_ticks, float* __restrict__ tick_obs = nullptr,
+                float* __restrict__ tick_links = nullptr) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t env = (int64_t)blockIdx.x * WARPS + warp;
+    if (env >= n) return;
+    WM& W = reinterpret_cast<WM*>(smem_raw)[warp];
+    env_step<WM, RAW>(W, lane, env, T, P, state, in, obs, rew, done, ticks, counters, n_ticks, tick_obs, tick_links);
 }
 

@@ -291,7 +291,8 @@ class SnakeVecEnv:
         """Checkpoint of the whole batch (the reference never checkpoints simulator state; SURVEY.md section 5):
         the [N,64] state array on the CPU plus the parameters' bytes.  With persistent manifolds on, also their warm-start
         factor (``manifold_warm``) and contact caches (``manifold_cache``, [N,1056] on the CPU), so that a restored batch
-        continues bit for bit.  With Bullet's literal tick on, ``bullet_tick_warm`` and the caches (``manifold_cache``)."""
+        continues bit for bit.  With Bullet's literal tick on, ``bullet_tick_warm`` and the caches (``manifold_cache``).  With the
+        joint-limit rows on, their angle (``joint_limit_angle``)."""
         sd = {"state": self.get_state().cpu(), "num_envs": self.num_envs, "params": bytes(self.params)}
         if getattr(self, "_manifold", None):
             sd["manifold_warm"] = self._manifold[1]
@@ -299,6 +300,8 @@ class SnakeVecEnv:
         if getattr(self, "_bullet", None) is not None:
             sd["bullet_tick_warm"] = self._bullet
             sd["manifold_cache"] = self.get_manifold_cache().cpu()
+        if getattr(self, "_limits", None) is not None:
+            sd["joint_limit_angle"] = self._limits
         return sd
 
     def _contact_model(self):
@@ -310,7 +313,8 @@ class SnakeVecEnv:
 
     def load_state_dict(self, sd):
         """Restore a :meth:`state_dict`.  Raises ``ValueError`` when the checkpoint comes from a batch with another size, other
-        parameters or another contact model (default, persistent manifolds, Bullet's literal tick, or another warm-start factor)."""
+        parameters, another contact model (default, persistent manifolds, Bullet's literal tick, or another warm-start factor) or
+        another joint-limit setting (off, or another angle); nothing is touched then."""
         if int(sd["num_envs"]) != self.num_envs or bytes(sd["params"]) != bytes(self.params):
             raise ValueError("checkpoint was taken from a batch with another size or other parameters")
         mine = self._contact_model()
@@ -319,6 +323,11 @@ class SnakeVecEnv:
         if mine != theirs:
             fmt = lambda m: m[0] if m[1] is None else "%s, warm %g" % m
             raise ValueError("checkpoint was taken with another contact model (%s; this batch: %s)" % (fmt(theirs), fmt(mine)))
+        lim_mine = getattr(self, "_limits", None)
+        lim_theirs = float(sd["joint_limit_angle"]) if "joint_limit_angle" in sd else None
+        if lim_mine != lim_theirs:
+            fmt = lambda a: "off" if a is None else "+-%g rad" % a
+            raise ValueError("checkpoint was taken with other joint limits (%s; this batch: %s)" % (fmt(lim_theirs), fmt(lim_mine)))
         if mine[1] is not None:
             self.set_manifold_cache(sd["manifold_cache"])  # checked before anything is touched
         self.set_state(sd["state"])
@@ -336,6 +345,23 @@ class SnakeVecEnv:
         to the handle's own solver.  Mirrors the oracle twin ``BulletTickOracle.set_bullet_tick`` (tests/); ``rollout_linear`` is refused while it is on."""
         _abi.check(self._lib.snk_set_bullet_tick(self._h, int(bool(on)), float(warm)), self._lib)
         self._bullet = float(warm) if on else None
+
+    def set_joint_limits(self, on=True, angle=1.57):
+        """Joint-limit rows (``snk_set_joint_limits``; PyBullet's btMultiBodyJointLimitConstraint, which loadURDF gives every
+        revolute joint of snake.urdf at +-1.57 rad): two unilateral rows per joint at +-``angle``, solved after the motor rows in
+        every sweep.  For the kernels with Bullet-order motor rows: ``motor_solver=0`` (or auto with a finite motor force) and
+        Bullet's literal tick (``set_bullet_tick``).  Refused on a handle with the exact motor solver unless the Bullet tick is on.
+        Off by default; mirrors ``Oracle.set_joint_limits``."""
+        self._check_open()
+        _abi.check(self._lib.snk_set_joint_limits(self._h, int(bool(on)), float(angle)), self._lib)
+        self._limits = float(angle) if on else None
+
+    def joint_limit_stats(self):
+        """(limit rows active at the end of a tick, summed over the environments and ticks of the last step launch, those ticks) --
+        ``snk_joint_limit_stats``; the oracle's ``row_stats()[1]`` counts the same rows."""
+        out = (ctypes.c_int64 * 2)()
+        _abi.check(self._lib.snk_joint_limit_stats(self._h, out), self._lib)
+        return int(out[0]), int(out[1])
 
     def get_manifold_cache(self):
         """The persistent manifolds' contact caches as a CUDA tensor [N, 1056] (``snk_get_manifold_cache``; layout in

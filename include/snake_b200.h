@@ -106,7 +106,8 @@ typedef struct snk_model {
 
 /* Task + solver parameters.  The defaults are the reference's task settings and PyBullet's documented world defaults (DESIGN.md
  * section 3).  The tick underneath is this project's restatement of Bullet, not Bullet itself -- one contact point per cylinder and
- * no persistent manifold (D1), no joint-limit / self-collision rows (D3), and with motor_solver = 2 the motor rows imposed exactly
+ * no persistent manifold (D1), no joint-limit / self-collision rows (D3: limit rows are a switch of the Bullet-order kernels,
+ * snk_set_joint_limits, off by default), and with motor_solver = 2 the motor rows imposed exactly
  * instead of relaxed by 50 sweeps (D4); DESIGN.md section 4 measures each.  No PyBullet was available to pin it against. */
 typedef struct snk_params {
     double dt;                  /* 1/240: Snake.setTimeSteps is never called (snake.py:271-272) */
@@ -219,8 +220,21 @@ int snk_set_manifold(snk_handle* h, int on, double warm_start);
  * warm_start: factor of the cached normal impulses that start the solver (Bullet: 0.1; 0 = off; < 0 is refused).  While it is on,
  * snk_step, snk_step_host*, snk_step_trace and snk_tick run the Bullet-tick kernel, the cache entry points and snk_manifold_stats
  * work, and snk_rollout_linear is refused.  Refused (SNK_E_ARG) while snk_set_manifold is on, and snk_set_manifold is refused while
- * this is on.  Synchronises the device. */
+ * this is on.  Synchronises the device.  on == 0 is refused on a handle with the exact motor solver while snk_set_joint_limits is on. */
 int snk_set_bullet_tick(snk_handle* h, int on, double warm_start);
+
+/* Joint-limit rows (btMultiBodyJointLimitConstraint, which pybullet.loadURDF gives every revolute joint of snake.urdf at +-1.57 rad):
+ * on != 0 adds two unilateral rows per joint at -angle and +angle to every kernel of this handle with Bullet-order motor rows -- the
+ * warp-per-env kernel when motor_solver resolves to 0, and Bullet's literal tick whenever snk_set_bullet_tick is on (either order).
+ * Every sweep solves them after the motor rows and before the contact rows; impulses >= 0, no warm start.  Inert while the joints stay
+ * inside the limits (outputs bit-identical to the rows off).  Refused (SNK_E_ARG) when angle is not a finite number > 0, and on a
+ * handle with the exact motor solver while the Bullet tick is off (its unlimited-force motor equalities admit no limit rows).  on == 0
+ * always succeeds.  Allocates nothing, does not synchronise; takes effect from the next launch. */
+int snk_set_joint_limits(snk_handle* h, int on, double angle);
+/* out[0] = joint-limit rows with a positive impulse at the end of a tick, summed over the environments and physics ticks of the last
+ * step launch; out[1] = those ticks (the oracle's row_stats()[1] counts the same rows).  SNK_E_ARG while the limits are off.
+ * Synchronises the device. */
+int snk_joint_limit_stats(snk_handle* h, int64_t out[2]);
 
 /* The contact caches of the persistent manifolds: SNK_MAN_STRIDE floats per environment, [N][SNK_MAN_STRIDE].  Cylinder c (0..31)
  * owns the floats [32 c, 32 c + 32): 4 slots of 8 words, slot s at 32 c + 8 s = (body-frame point x, y, z, distance to the ground
