@@ -613,6 +613,10 @@ __device__ __forceinline__ void man_run(const KParams& P, float* __restrict__ st
         if (fin) {
             ExStepOut o;
             ex_step_end(cT, P, e, run, &o);
+            if (o.bad) { // force-reset: the environment restarts like a hard reset, its caches (impulses of this step not finite) emptied
+#pragma unroll 1
+                for (int k = 0; k < MAN_STRIDE; k += 4) *reinterpret_cast<float4*>(mc + k) = make_float4(0.f, 0.f, 0.f, 0.f);
+            }
             if (ROLL) {
                 c_ticks += (unsigned long long)o.ticks; c_iters += (unsigned long long)o.iters; c_done += o.done; c_bad += o.bad;
                 ret = (t == 0) ? o.rew : ret + o.rew;

@@ -600,7 +600,12 @@ __device__ __forceinline__ void bt_env_step(WarpMemBt& W, int lane, int64_t env,
     if (bad) { d = true; r = P.donepen; }
     else if (d) r += P.donepen;
     __syncwarp();
-    if (bad) { W.s[lane] = 0.f; W.s[lane + 32] = 0.f; __syncwarp(); }
+    if (bad) { // force-reset: the environment restarts like a hard reset, its caches (impulses of this step not finite) emptied
+        W.s[lane] = 0.f; W.s[lane + 32] = 0.f;
+#pragma unroll 1
+        for (int k = 4 * lane; k < SNK_MAN_STRIDE; k += 128) *reinterpret_cast<float4*>(mc + k) = make_float4(0.f, 0.f, 0.f, 0.f);
+        __syncwarp();
+    }
     if (lane == 0) { W.s[SNK_S_RET] += r; W.s[SNK_S_LEN] += 1.f; }
     __syncwarp();
     if (d) { soft_reset(W, P, lane); __syncwarp(); } // in-step reset + worker reset: post-reset obs (multiprocessing_env.py:14-15)

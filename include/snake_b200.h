@@ -208,8 +208,9 @@ int snk_rollout_linear(snk_handle* h, const float* weights_dev, const float* mea
  * the cached normal impulses x warm_start (Bullet: 0.1; 0 = off) start the solver.  The call (re)allocates and CLEARS the caches
  * (4 224 B per environment + 388 MB of row tables per device); they survive soft resets like Bullet's (Q10).  on == 0 returns to
  * the default one-point-per-cylinder tick (deviation D1) and frees the memory.  Only with the exact motor solver.  While it is on,
- * snk_step, snk_step_host*, snk_step_trace and snk_rollout_linear run the manifold kernels; snk_tick is refused.  Synchronises the
- * device. */
+ * snk_step, snk_step_host*, snk_step_trace and snk_rollout_linear run the manifold kernels; snk_tick is refused.  An environment
+ * whose state goes non-finite in an env-step (counter word 3 of snk_last_counters) restarts like a hard reset: its caches are emptied
+ * with the force-reset, so no cached impulse of that step warm-starts the next one.  Synchronises the device. */
 int snk_set_manifold(snk_handle* h, int on, double warm_start);
 
 /* Bullet's literal tick: Bullet-order motor rows (relaxed inside the projected Gauss-Seidel, as with motor_solver = 0) together with
@@ -219,8 +220,9 @@ int snk_set_manifold(snk_handle* h, int on, double warm_start);
  * the caches (4 224 B per environment, layout SNK_MAN_STRIDE below); on == 0 frees them and returns to the handle's own solver.
  * warm_start: factor of the cached normal impulses that start the solver (Bullet: 0.1; 0 = off; < 0 is refused).  While it is on,
  * snk_step, snk_step_host*, snk_step_trace and snk_tick run the Bullet-tick kernel, the cache entry points and snk_manifold_stats
- * work, and snk_rollout_linear is refused.  Refused (SNK_E_ARG) while snk_set_manifold is on, and snk_set_manifold is refused while
- * this is on.  Synchronises the device.  on == 0 is refused on a handle with the exact motor solver while snk_set_joint_limits is on. */
+ * work, and snk_rollout_linear is refused.  A non-finite force-reset empties that environment's caches, as with snk_set_manifold
+ * (snk_tick has no non-finite check and leaves them).  Refused (SNK_E_ARG) while snk_set_manifold is on, and snk_set_manifold is refused
+ * while this is on.  Synchronises the device.  on == 0 is refused on a handle with the exact motor solver while snk_set_joint_limits is on. */
 int snk_set_bullet_tick(snk_handle* h, int on, double warm_start);
 
 /* Joint-limit rows (btMultiBodyJointLimitConstraint, which pybullet.loadURDF gives every revolute joint of snake.urdf at +-1.57 rad):
@@ -284,7 +286,8 @@ int snk_set_state(snk_handle* h, const float* state_dev, void* stream);
 
 /* Per-launch counters of the last snk_step (device-side sums, read back synchronously):
  * out[0] = total physics ticks, out[1] = total PGS iterations, out[2] = dones,
- * out[3] = environments whose state went non-finite and were force-reset. */
+ * out[3] = environments whose state went non-finite and were force-reset: done with reward done_penalty and the reset pose, and
+ *          with persistent manifolds on (snk_set_manifold, snk_set_bullet_tick) their contact caches emptied, as a hard reset does. */
 int snk_last_counters(snk_handle* h, int64_t out[4]);
 
 /* Number of kernels this library has launched on this handle since creation. */

@@ -243,7 +243,10 @@ static void bt_env_step(Handle* h, int64_t* cnt, real* s, const real* action, re
     real r = P->alpha * (o[48] - xprev) + ((FABS(o[55]) > P->colf) ? P->colpen : 0) - P->beta * FABS(o[49] - 0) - P->gamma * energy;
     /* checkTermination (SnakeGymEnv.py:99-103) */
     int d = (FABS(o[P->tjoint]) > P->tang) || (K.height > P->hthr) || end_height;
-    if (bad) { d = 1; r = P->donepen; cnt[3] += 1; for (int k = 0; k < SNK_STATE_STRIDE; k++) s[k] = 0; s[SNK_S_QUAT + 3] = 1; }
+    if (bad) { /* force-reset: restarts like a hard reset, contact caches emptied (their impulses of this step are not finite) */
+        d = 1; r = P->donepen; cnt[3] += 1; for (int k = 0; k < SNK_STATE_STRIDE; k++) s[k] = 0; s[SNK_S_QUAT + 3] = 1;
+        if (h->M) memset(h->M + ((s - h->S) / SNK_STATE_STRIDE) * NC, 0, NC * sizeof(Manifold));
+    }
     else if (d) r += P->donepen;
     s[SNK_S_RET] += r; s[SNK_S_LEN] += 1;
     if (d) { /* in-step reset + worker reset: returned obs is the post-reset one */
